@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--steps K] [--warmup W]      # CPU restatement of the reference path
+    python bench.py --steps K --dump-outputs DIR                   # + the last timed step's outputs as DIR/<name>.npy
 
 One step = forward (p_m, p_v, inside_elbo_recon/kl, ce_term) + backward of
 J = KL_term + <g_m, p_m> + <g_v, p_v> to y, noise, inducing points and kernel hypers, on the SWEEP
@@ -51,7 +52,13 @@ def parse():
     ap.add_argument("--lean", action="store_true", help="big configurations on a GPU budget: no extra profiling step (the per-kernel / collective "
                     "profile is taken on the last timed step's twin run only when not lean: here on the first warm-up step) and no e2e loop")
     ap.add_argument("--strong", action="store_true", help="strong scaling: --n is the TOTAL number of datapoints, split over the GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (p_m, p_v, the "
+                    "ELBO terms, mu_hat, A_hat, the gradients of y, noise and the parameters) to DIR/<name>.npy; large arrays are "
+                    "cut to fixed, seeded samples so that the dump stays below 64 MB (rank 0's rows on several GPUs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # --------------------------------------------------------------------------------------------------
@@ -263,6 +270,36 @@ def measure_f16_peak(dev):
     return best
 
 
+DUMP_BYTES = 48 << 20                 # array data of --dump-outputs: the files, headers included, stay well below 64 MB
+DUMP_WHOLE_BYTES = 1 << 20            # arrays up to this size are always written whole
+
+
+def dump_outputs(out_dir, arrays, n_rows):
+    """Write each tensor of `arrays` to out_dir/<name>.npy, float64 ones as float64 and all others as float32, at most
+    DUMP_BYTES of array data in all.  Arrays of up to DUMP_WHOLE_BYTES are written whole; when the others do not fit in
+    what is left, each of them keeps the same fraction of itself: arrays with one row per datapoint a sample of rows
+    (seed 0, ascending, the same rows for all of them), any other array a sample of its flattened elements (seed 0,
+    ascending).  The samples depend only on the shapes, so two builds run with the same arguments can be compared array
+    for array."""
+    import numpy as np
+    arrays = {k: v.detach() if v.dtype == torch.float64 else v.detach().float() for k, v in arrays.items()}
+    nbytes = lambda v: v.numel() * v.element_size()
+    large = {k for k, v in arrays.items() if nbytes(v) > DUMP_WHOLE_BYTES}
+    room = DUMP_BYTES - sum(nbytes(v) for k, v in arrays.items() if k not in large)
+    frac = min(1.0, room / max(1, sum(nbytes(arrays[k]) for k in large)))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        if k in large and frac < 1.0:
+            g = torch.Generator().manual_seed(0)
+            if v.shape[0] == n_rows:
+                idx = torch.randperm(n_rows, generator=g)[:int(n_rows * frac)].sort().values
+                v = v.index_select(0, idx.to(v.device))
+            else:
+                idx = torch.randint(v.numel(), (int(v.numel() * frac),), generator=g).unique()     # sorted, at most that many
+                v = v.reshape(-1).index_select(0, idx.to(v.device))
+        np.save(os.path.join(out_dir, k + ".npy"), v.cpu().numpy())
+
+
 def run_gpu(args):
     import torch.distributed as dist
     import svgp_vae_b200 as pkg
@@ -331,7 +368,11 @@ def run_gpu(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()) / steps
 
-    dev_step = lambda: step(aux, y.detach(), noise.detach())
+    last = []                                                    # outputs of the latest step, for --dump-outputs
+
+    def dev_step():
+        last.clear()                                             # released before the next step allocates its own
+        last.append(step(aux, y.detach(), noise.detach()))
     from svgp_vae_b200 import step as step_mod
     prof, coll = None, {}
     for w in range(args.warmup):
@@ -347,6 +388,13 @@ def run_gpu(args):
     with ClockSampler(local) as clocks:
         ms = timed(dev_step, args.steps)
     launches = (be.launches - l0) // max(args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        res, gy, gn = last[0]
+        arrays = {k: v for k, v in res.items() if isinstance(v, torch.Tensor)}
+        arrays.update(grad_y=gy, grad_noise=gn)
+        arrays.update(("grad_" + k, p.grad) for k, p in svgp.named_parameters() if p.grad is not None)
+        dump_outputs(args.dump_outputs, arrays, N)
+    last.clear()
 
     # per-kernel device times of one more step (CUDA events on the launch stream)
     if prof is None:
@@ -356,6 +404,7 @@ def run_gpu(args):
         dev_step()
         prof = be.stop_profile()
         coll = step_mod.stop_coll_profile() if world > 1 else {}
+        last.clear()
 
     # e2e: pinned host buffers in, results out, every step
     if args.lean:
