@@ -41,6 +41,10 @@ extern "C" {
 #define SVGP_K_EXPSIN 2 /* tfk.ExpSinSquared, period 2*pi: s^2 exp(-2 sum sin^2((x-z)/2)/l^2)  */
 #define SVGP_K_LINEAR 3 /* tfk.Linear(): x . z                                                */
 #define SVGP_K_COSINE 4 /* Linear divided by |x||z|  (K_obj_normalize)                        */
+/* Matern factors, tfk.MaternOneHalf / MaternThreeHalves / MaternFiveHalves: r = |x-z| over the block, u = c r / l   */
+#define SVGP_K_MATERN12 5 /* s^2 exp(-u), c = 1; its gradient in x and z is taken as 0 at r = 0 (symmetric subgradient) */
+#define SVGP_K_MATERN32 6 /* s^2 (1 + u) exp(-u), c = sqrt(3)                                                     */
+#define SVGP_K_MATERN52 7 /* s^2 (1 + u + u^2/3) exp(-u), c = sqrt(5)                                             */
 
 /* implementation selector for the GEMM-class entry points */
 #define SVGP_IMPL_AUTO 0

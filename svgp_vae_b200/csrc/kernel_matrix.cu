@@ -3,7 +3,8 @@
 // spritesSVGP.kernel_matrix (:550-600), the ball's kernel.matrix calls (:81-86, :152-157)
 // and the tfp.math.psd_kernels arithmetic under them (formulas: oracle/tfp_kernels.py).
 //
-// k(x, z) = kA(xA, zA) * kB(xB, zB), each factor one of NONE / SE / EXPSIN / LINEAR / COSINE.
+// k(x, z) = kA(xA, zA) * kB(xB, zB), each factor one of NONE / SE / EXPSIN / LINEAR / COSINE / MATERN12 / MATERN32 /
+// MATERN52.
 // The builder is HBM-bound: every output element is written once (coalesced, through a
 // padded shared-memory tile so that both K (N x M) and its transpose Kt (M x N) leave the SM
 // as full row segments), optionally as a scaled fp16 hi/lo pair for the tcgen05 consumers.
@@ -51,6 +52,20 @@ __device__ __forceinline__ Hyp load_hyp(const float* hyp) {
   return h;
 }
 
+// Matern factors: k = a^2 p(u) e^-u with u = c r / l, r = |x - z| over the block, c = 1, sqrt 3, sqrt 5 and
+// p(u) = 1, 1 + u, 1 + u + u^2 / 3 for nu = 1/2, 3/2, 5/2
+__host__ __device__ __forceinline__ bool is_matern(int type) {
+  return type == SVGP_K_MATERN12 || type == SVGP_K_MATERN32 || type == SVGP_K_MATERN52;
+}
+__device__ __forceinline__ float matern_c(int type) {
+  return type == SVGP_K_MATERN12 ? 1.0f : (type == SVGP_K_MATERN32 ? 1.7320508075688772f : 2.2360679774997897f);
+}
+__device__ __forceinline__ float matern_poly(int type, float u) {
+  if (type == SVGP_K_MATERN12) return 1.0f;
+  if (type == SVGP_K_MATERN32) return 1.0f + u;
+  return fmaf(u, u * (1.0f / 3.0f), 1.0f + u);
+}
+
 // value of one factor.  nx / nz are the Euclidean norms of the feature blocks (COSINE only).
 __device__ __forceinline__ float factor_value(int type, const float* x, const float* z, int d, float amp,
                                               float len, float nx, float nz) {
@@ -64,6 +79,12 @@ __device__ __forceinline__ float factor_value(int type, const float* x, const fl
     float u = 0.f;
     for (int f = 0; f < d; ++f) { float s = sinf(0.5f * fabsf(x[f] - z[f])); u = fmaf(s, s, u); }
     return amp * amp * expf(-2.0f * u / (len * len));
+  }
+  if (is_matern(type)) {
+    float r2 = 0.f;
+    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; r2 = fmaf(t, t, r2); }
+    const float u = matern_c(type) * sqrtf(r2) / len;
+    return amp * amp * matern_poly(type, u) * expf(-u);
   }
   float dot = 0.f;
   for (int f = 0; f < d; ++f) dot = fmaf(x[f], z[f], dot);
@@ -86,6 +107,14 @@ __device__ __forceinline__ double factor_value_f64(int type, const float* x, con
     double u = 0.0;
     for (int f = 0; f < d; ++f) { const double s = sin(0.5 * fabs((double)x[f] - (double)z[f])); u = fma(s, s, u); }
     return amp * amp * exp(-2.0 * u / (len * len));
+  }
+  if (is_matern(type)) {
+    double r2 = 0.0;
+    for (int f = 0; f < d; ++f) { const double t = (double)x[f] - (double)z[f]; r2 = fma(t, t, r2); }
+    const double c = type == SVGP_K_MATERN12 ? 1.0 : (type == SVGP_K_MATERN32 ? 1.7320508075688772 : 2.23606797749979);
+    const double u = c * sqrt(r2) / len;
+    const double p = type == SVGP_K_MATERN12 ? 1.0 : (type == SVGP_K_MATERN32 ? 1.0 + u : fma(u, u * (1.0 / 3.0), 1.0 + u));
+    return amp * amp * p * exp(-u);
   }
   double dot = 0.0;
   for (int f = 0; f < d; ++f) dot = fma((double)x[f], (double)z[f], dot);
@@ -130,6 +159,32 @@ __device__ __forceinline__ FactorAdj factor_adjoint(int type, const float* x, co
     a.c1 = gk / (nx * nz);
     a.c2z = -gk * kval / (nz * nz);
     a.c2x = -gk * kval / (nx * nx);
+  } else if (is_matern(type)) {
+    // dk/dz_f = C (x_f - z_f) with C = -(dk/du) c / (l r); written with e = a^2 e^-u = kval / p(u), C stays finite at r = 0
+    // for nu = 3/2, 5/2 and no division by r appears.  nu = 1/2 has C = k / (l r): 0 at r = 0 (the symmetric subgradient,
+    // which gives the exact total derivative of k(z, z) = a^2 when both sides are summed, as the K_mm adjoint does)
+    float r2 = 0.f;
+    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; r2 = fmaf(t, t, r2); }
+    const float r = sqrtf(r2), u = matern_c(type) * r / len;
+    const float il2 = 1.0f / (len * len);
+    float C, dl;
+    if (type == SVGP_K_MATERN12) {
+      C = r > 0.f ? kval / (len * r) : 0.f;
+      dl = kval * u / len;                                    // dk/dl = k u / l
+    } else if (type == SVGP_K_MATERN32) {
+      const float e = kval / (1.0f + u);
+      C = 3.0f * e * il2;
+      dl = e * u * u / len;                                   // dk/dl = a^2 u^2 e^-u / l
+    } else {
+      const float p1 = 1.0f + u, e = kval / fmaf(u, u * (1.0f / 3.0f), p1);
+      C = (5.0f / 3.0f) * p1 * e * il2;
+      dl = e * (u * u * (1.0f / 3.0f)) * p1 / len;            // dk/dl = a^2 e^-u (u^2 / 3)(1 + u) / l
+    }
+    a.c1 = gk * C;
+    a.c2z = -a.c1;
+    a.c2x = -a.c1;
+    a.damp = gk * 2.0f * kval / amp;
+    a.dlen = gk * dl;
   }
   return a;
 }
@@ -170,9 +225,9 @@ __device__ __forceinline__ void load_features(const float* F, int64_t ld, int64_
 // max|x| max|z| for LINEAR, 1 for COSINE) is brought just below 2^14, so that value * scale = hi + lo keeps
 // 22 significand bits for every entry larger than 2^-17 of the bound and never overflows fp16.
 __device__ __forceinline__ float factor_bound(int type, float amp, float nx, float nz) {
-  if (type == SVGP_K_SE || type == SVGP_K_EXPSIN) return amp * amp;
   if (type == SVGP_K_LINEAR) return nx * nz;
-  return 1.0f;
+  if (type == SVGP_K_NONE || type == SVGP_K_COSINE) return 1.0f;
+  return amp * amp;                    // SE, EXPSIN and the Matern factors
 }
 __device__ __forceinline__ float plane_scale(Spec sp, Hyp h, const float* ks) {
   float b = factor_bound(sp.ta, h.amp_a, ks[2], ks[4]) * factor_bound(sp.tb, h.amp_b, ks[3], ks[5]);
@@ -187,7 +242,7 @@ __device__ __forceinline__ float plane_scale(Spec sp, Hyp h, const float* ks) {
 
 // every entry of K is >= 0 (stationary factors only): recorded in kscale[6] for the SYRK's truncation-bias correction
 __device__ __forceinline__ bool kernel_nonneg(Spec sp) {
-  auto ok = [](int t) { return t == SVGP_K_NONE || t == SVGP_K_SE || t == SVGP_K_EXPSIN; };
+  auto ok = [](int t) { return t != SVGP_K_LINEAR && t != SVGP_K_COSINE; };   // (check_spec admits nothing else)
   return ok(sp.ta) && ok(sp.tb);
 }
 
@@ -657,12 +712,15 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
 //   pass X: one block per row tile walks every column tile      -> dFx rows (plain stores)
 //   pass Z: one block per (column tile, row slab) walks its rows -> dFz, dhyp (double atomics,
 //           one flush per block)
+// ACC64 (pass Z of the Matern factors): the per-tile fp32 partials are folded into double across the row tiles and the
+// flush  dz_f = sum c1 x_f + z_f sum c2z  (which cancels: c2z = -c1) is done in double, as in kernel_bwd_z_se44_kernel
 // ------------------------------------------------------------------------------------------
-template <bool PASS_X>
+template <bool PASS_X, bool ACC64 = false>
 __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
     const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz, int64_t M,
     Spec sp, const float* __restrict__ hyp, const float* __restrict__ G, int64_t ldg, float* __restrict__ dFx,
     double* __restrict__ dFz, double* __restrict__ dhyp) {
+  static_assert(!(PASS_X && ACC64), "ACC64 is a Z-pass variant");
   extern __shared__ float smem[];
   const int d = sp.da + sp.db, dp = d | 1;
   float* xs = smem;
@@ -688,6 +746,9 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
 #pragma unroll
     for (int q = 0; q < MAXD / 4; ++q) acc[q] = 0.f;
     float own_acc[4] = {0.f, 0.f, 0.f, 0.f};
+    double acc64[ACC64 ? MAXD / 4 : 1], own64[4] = {0.0, 0.0, 0.0, 0.0};
+#pragma unroll
+    for (int q = 0; q < (ACC64 ? MAXD / 4 : 1); ++q) acc64[q] = 0.0;
     // hyper-parameter gradients are heavily cancelling sums over all N x M entries: accumulate them in double
     double hy[4] = {0.0, 0.0, 0.0, 0.0};
     if (threadIdx.x < 4) hred[threadIdx.x] = 0.f;
@@ -745,10 +806,14 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
             } else {
               for (int k = 0; k < TILE; ++k) s = fmaf(cmat[k * (TILE + 1) + o], xs[k * dp + f], s);
             }
-            acc[q] += s;
+            if (ACC64) acc64[q] += (double)s;
+            else acc[q] += s;
           }
         }
-        if (fg == 0) {
+        if (ACC64) {          // every thread keeps its own copy: the flush needs no broadcast
+          own64[0] += (double)own[o * 4 + 0]; own64[1] += (double)own[o * 4 + 1];
+          own64[2] += (double)own[o * 4 + 2]; own64[3] += (double)own[o * 4 + 3];
+        } else if (fg == 0) {
           own_acc[0] += own[o * 4 + 0]; own_acc[1] += own[o * 4 + 1];
           own_acc[2] += own[o * 4 + 2]; own_acc[3] += own[o * 4 + 3];
         }
@@ -768,6 +833,13 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
         const int f = fg + 4 * q;
         if (f >= d) continue;
         bool inA = f < sp.da;
+        if (ACC64) {
+          double v = acc64[q] + own64[inA ? 0 : 1] * (double)self[f];
+          if (inA && f == 0 && sp.ta == SVGP_K_EXPSIN) v += own64[2];
+          if (!inA && f == sp.da && sp.tb == SVGP_K_EXPSIN) v += own64[3];
+          if (go < M) atomicAdd(&dFz[go * d + f], v);
+          continue;
+        }
         float v = acc[q] + own[o * 4 + (inA ? 0 : 1)] * self[f];
         // EXPSIN contributes only through its single feature (the first of its block)
         if (inA && f == 0 && sp.ta == SVGP_K_EXPSIN) v += own[o * 4 + 2];
@@ -982,7 +1054,7 @@ static size_t bwd_smem(int d) {
 
 static int check_spec(int ta, int da, int tb, int db) {
   auto ok = [](int t, int d) {
-    if (t < 0 || t > 4 || d < 0) return false;
+    if (t < 0 || t > SVGP_K_MATERN52 || d < 0) return false;
     if (t == SVGP_K_NONE) return d == 0;
     if (t == SVGP_K_EXPSIN) return d == 1;
     return d >= 1;
@@ -1152,6 +1224,8 @@ int svgp_kernel_bwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
                       !getenv("SVGP_K1_BWD_GENERIC");
     if (se44)
       kernel_bwd_z_se44_kernel<<<grid, THREADS, 0, st>>>(Fx, ldx, N, Fz, ldz, M, hyp, G, ldg, dFz, dhyp);
+    else if (is_matern(type_a) || is_matern(type_b))
+      kernel_bwd_kernel<false, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
     else
       kernel_bwd_kernel<false><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
     int rc = check_launch("svgp_kernel_bwd(z)");

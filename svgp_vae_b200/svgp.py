@@ -19,7 +19,8 @@ import numpy as np
 import torch
 
 from . import ops
-from ._lib import SVGP_K_COSINE, SVGP_K_EXPSIN, SVGP_K_LINEAR, SVGP_K_NONE, SVGP_K_SE
+from ._lib import (SVGP_K_COSINE, SVGP_K_EXPSIN, SVGP_K_LINEAR, SVGP_K_MATERN12, SVGP_K_MATERN32, SVGP_K_MATERN52,
+                   SVGP_K_NONE, SVGP_K_SE)
 from .step import LOG_2PI, elbo_terms, svgp_step
 
 
@@ -317,9 +318,20 @@ class productSVGP(mainSVGP):
     """Continuous two-block product kernel kA(x[:, :dA], z[:, :dA]) * kB(x[:, dA:], z[:, dA:]) with data rows laid
     out like inducing rows (no id column).  Not in the reference: it is the full-rank stand-in the synthetic sweeps
     need (SURVEY H3: the MNIST kernel is rank-deficient beyond M ~ 64); with SE x SE it is spritesSVGP's K_SE form
-    (:542-544) without the action-id gather."""
+    (:542-544) without the action-id gather.
 
-    _TYPES = {"se": SVGP_K_SE, "linear": SVGP_K_LINEAR, "cosine": SVGP_K_COSINE, "none": SVGP_K_NONE}
+    ``kind_a`` / ``kind_b`` name each factor: "se" (tfk.ExponentiatedQuadratic), "matern12", "matern32", "matern52"
+    (tfk.MaternOneHalf / MaternThreeHalves / MaternFiveHalves: a^2 p(u) exp(-u), u = c |x - z| / l with c = 1, sqrt 3,
+    sqrt 5), "linear", "cosine" or "none" (a factor of 1; its block must be empty).  Every stationary factor takes its
+    own amplitude a and length scale l from ``amplitude`` / ``length_scale``.  The Matern kinds suit rough continuous
+    auxiliary data (time, position, pose), where SE's infinitely smooth prior is too strong; e.g. a Matern 3/2 kernel
+    over time times a Matern 5/2 kernel over a 3-D position:
+
+        productSVGP(Z, dim_a=1, dim_b=3, kind_a="matern32", kind_b="matern52", N_train=N, L=L)
+    """
+
+    _TYPES = {"se": SVGP_K_SE, "linear": SVGP_K_LINEAR, "cosine": SVGP_K_COSINE, "none": SVGP_K_NONE,
+              "matern12": SVGP_K_MATERN12, "matern32": SVGP_K_MATERN32, "matern52": SVGP_K_MATERN52}
 
     def __init__(self, initial_inducing_points, dim_a, dim_b, name="prod", jitter=1e-2, N_train=1, L=1, kind_a="se",
                  kind_b="se", amplitude=(1.0, 1.0), length_scale=(1.0, 1.0), fixed_inducing_points=False,
