@@ -45,6 +45,9 @@ extern "C" {
 #define SVGP_K_MATERN12 5 /* s^2 exp(-u), c = 1; its gradient in x and z is taken as 0 at r = 0 (symmetric subgradient) */
 #define SVGP_K_MATERN32 6 /* s^2 (1 + u) exp(-u), c = sqrt(3)                                                     */
 #define SVGP_K_MATERN52 7 /* s^2 (1 + u + u^2/3) exp(-u), c = sqrt(5)                                             */
+/* automatic relevance determination: OR'ed into SVGP_K_SE or a Matern code, the factor's distance becomes
+ * r^2 = sum_f ((x_f - z_f) / l_f)^2 with one length scale l_f per feature column of its block (hyp layout below)      */
+#define SVGP_K_ARD 16
 
 /* implementation selector for the GEMM-class entry points */
 #define SVGP_IMPL_AUTO 0
@@ -69,6 +72,10 @@ int svgp_device_ok(void);          /* 1 if the current device is compute capabil
  *           .matrix/.apply calls under them.
  * Fx (N x d) / Fz (M x d) are dense fp32 feature rows [block A | block B], d = dim_a+dim_b.
  * hyp = device float[4] = {amplitude_a, length_a, amplitude_b, length_b} (unused entries 1).
+ * With SVGP_K_ARD on either factor hyp = device float[4 + dim_a + dim_b]: hyp[4 + f] is the length scale of feature
+ * column f of the [A | B] row.  An ARD block reads its l_f there and not its isotropic slot (hyp[1] / hyp[3]); an
+ * isotropic block reads its slot and not its hyp[4 + f] (callers put 1 there).  The type codes may carry the flag in
+ * every K1 entry point below.
  * Outputs (each group may be NULL):
  *   K   (N x M fp32, ld = ldk)                         plain matrix for the SIMT consumers; requested alone and with
  *                                                      N M <= 2^26 it is the float64 evaluation rounded once to fp32
@@ -86,7 +93,9 @@ int svgp_kernel_fwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
                     int64_t ldkt, float* kscale, void* stream);
 
 /* adjoint of svgp_kernel_fwd.  G (N x M) is dObjective/dK.  dFx (N x d) is overwritten;
- * dFz (M x d, double) and dhyp (double[4]) are ACCUMULATED into (caller zeroes them).
+ * dFz (M x d, double) and dhyp (double[4], double[4 + dim_a + dim_b] for ARD specs: slot 4 + f takes dObjective/dl_f,
+ * and the slots hyp does not read get exactly 0) are ACCUMULATED into (caller zeroes them).  The same for
+ * svgp_kernel_diag_bwd.
  * replaces: tf.gradients through kernel_matrix (MNIST_experiment.py:202-208).                */
 int svgp_kernel_bwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, int64_t ldz, int64_t M,
                     int type_a, int dim_a, int type_b, int dim_b, const float* hyp,

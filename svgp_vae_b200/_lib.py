@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_HERE, "libsvgp_b200.so")
 
 SVGP_K_NONE, SVGP_K_SE, SVGP_K_EXPSIN, SVGP_K_LINEAR, SVGP_K_COSINE = 0, 1, 2, 3, 4
 SVGP_K_MATERN12, SVGP_K_MATERN32, SVGP_K_MATERN52 = 5, 6, 7
+SVGP_K_ARD = 16       # OR'ed into SE / Matern codes: one length scale per feature column (include/svgp_b200.h)
 IMPL_AUTO, IMPL_SIMT, IMPL_TC, IMPL_TC_I8, IMPL_TC_I8_D3, IMPL_TC_I8_O4 = 0, 1, 2, 3, 4, 5
 
 

@@ -246,7 +246,7 @@ class CudaBackend:
         ta, da, tb, db = spec
         dFx = torch.empty((N, d), device=Fx.device, dtype=torch.float32) if need_x else None
         dFz = torch.zeros((M, d), device=Fx.device, dtype=torch.float64) if need_z else None
-        dhyp = torch.zeros(4, device=Fx.device, dtype=torch.float64)
+        dhyp = torch.zeros(hyp.numel(), device=Fx.device, dtype=torch.float64)     # 4 + d for ARD specs
         _call("svgp_kernel_bwd", _ptr(Fx), Fx.stride(0), N, _ptr(Fz), Fz.stride(0), M, ta, da, tb, db, _ptr(hyp),
                   _ptr(G), G.stride(0), _ptr(dFx), _ptr(dFz), _ptr(dhyp), _stream())
         self.launches += int(need_x) + int(need_z)
@@ -265,7 +265,7 @@ class CudaBackend:
         Fx, Fy, hyp, g = _f32c(Fx), _f32c(Fy), _f32c(hyp), _f32c(g)
         ta, da, tb, db = spec
         dFx, dFy = torch.empty_like(Fx), torch.empty_like(Fy)
-        dhyp = torch.zeros(4, device=Fx.device, dtype=torch.float64)
+        dhyp = torch.zeros(hyp.numel(), device=Fx.device, dtype=torch.float64)
         _call("svgp_kernel_diag_bwd", _ptr(Fx), Fx.stride(0), _ptr(Fy), Fy.stride(0), Fx.shape[0], ta, da, tb, db,
                   _ptr(hyp), _ptr(g), _ptr(dFx), _ptr(dFy), _ptr(dhyp), _stream())
         self.launches += 1

@@ -38,8 +38,10 @@ const char* last_error() { return g_err; }
 // ------------------------------------------------------------------------------------------
 // factor arithmetic
 // ------------------------------------------------------------------------------------------
+// ta / tb are the base type codes: the SVGP_K_ARD flag is stripped at the ABI boundary into ard_a / ard_b
 struct Spec {
   int ta, da, tb, db;
+  bool ard_a, ard_b;
 };
 
 struct Hyp {
@@ -67,12 +69,15 @@ __device__ __forceinline__ float matern_poly(int type, float u) {
 }
 
 // value of one factor.  nx / nz are the Euclidean norms of the feature blocks (COSINE only).
+// ARD: the SE and Matern distances take every difference times il[f], the inverse length scale of feature f (1 on the
+// features of an isotropic block, whose len is its own; len = 1 for an ARD block)
+template <bool ARD = false>
 __device__ __forceinline__ float factor_value(int type, const float* x, const float* z, int d, float amp,
-                                              float len, float nx, float nz) {
+                                              float len, float nx, float nz, const float* il = nullptr) {
   if (type == SVGP_K_NONE) return 1.0f;
   if (type == SVGP_K_SE) {
     float r2 = 0.f;
-    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; r2 = fmaf(t, t, r2); }
+    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; if (ARD) t *= il[f]; r2 = fmaf(t, t, r2); }
     return amp * amp * expf(-0.5f * r2 / (len * len));
   }
   if (type == SVGP_K_EXPSIN) {
@@ -82,7 +87,7 @@ __device__ __forceinline__ float factor_value(int type, const float* x, const fl
   }
   if (is_matern(type)) {
     float r2 = 0.f;
-    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; r2 = fmaf(t, t, r2); }
+    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; if (ARD) t *= il[f]; r2 = fmaf(t, t, r2); }
     const float u = matern_c(type) * sqrtf(r2) / len;
     return amp * amp * matern_poly(type, u) * expf(-u);
   }
@@ -95,12 +100,14 @@ __device__ __forceinline__ float factor_value(int type, const float* x, const fl
 // the same in float64 arithmetic on the fp32 features (the integer tensor-core operands and the M x M stage's K_mm:
 // an fp32 evaluation carries ~|exponent| 2^-24 ~ 5e-7 of relative error per entry, which the ill-conditioned M x M
 // stage turns into 1e-4 of the inducing-point gradient at M = 2048 -- tools/numerics/sim_parity.py, SIM_KNOISE)
+// (ARD: the exact float64 difference times the float64 inverse length scale -- no rounding of x_f / l_f to fp32)
+template <bool ARD = false>
 __device__ __forceinline__ double factor_value_f64(int type, const float* x, const float* z, int d, double amp,
-                                                   double len, double nx, double nz) {
+                                                   double len, double nx, double nz, const double* il = nullptr) {
   if (type == SVGP_K_NONE) return 1.0;
   if (type == SVGP_K_SE) {
     double r2 = 0.0;
-    for (int f = 0; f < d; ++f) { const double t = (double)x[f] - (double)z[f]; r2 = fma(t, t, r2); }
+    for (int f = 0; f < d; ++f) { double t = (double)x[f] - (double)z[f]; if (ARD) t *= il[f]; r2 = fma(t, t, r2); }
     return amp * amp * exp(-0.5 * r2 / (len * len));
   }
   if (type == SVGP_K_EXPSIN) {
@@ -110,7 +117,7 @@ __device__ __forceinline__ double factor_value_f64(int type, const float* x, con
   }
   if (is_matern(type)) {
     double r2 = 0.0;
-    for (int f = 0; f < d; ++f) { const double t = (double)x[f] - (double)z[f]; r2 = fma(t, t, r2); }
+    for (int f = 0; f < d; ++f) { double t = (double)x[f] - (double)z[f]; if (ARD) t *= il[f]; r2 = fma(t, t, r2); }
     const double c = type == SVGP_K_MATERN12 ? 1.0 : (type == SVGP_K_MATERN32 ? 1.7320508075688772 : 2.23606797749979);
     const double u = c * sqrt(r2) / len;
     const double p = type == SVGP_K_MATERN12 ? 1.0 : (type == SVGP_K_MATERN32 ? 1.0 + u : fma(u, u * (1.0 / 3.0), 1.0 + u));
@@ -131,15 +138,19 @@ __device__ __forceinline__ double block_norm_f64(const float* v, int d) {
 //   d/dz_f = c1 * x_f + c2z * z_f (+ e for EXPSIN on its single feature, sign + for z, - for x)
 //   d/dx_f = c1 * z_f + c2x * x_f
 //   d/d amp, d/d len returned through damp / dlen
+// ARD: the coefficients are those of the scaled coordinates x_f il_f, z_f il_f (len = 1 for an ARD block): on the
+// unscaled features d/dz_f = il_f^2 (c1 x_f + c2z z_f), d/dl_f = il_f^3 c1 (x_f - z_f)^2, and dlen means nothing
 struct FactorAdj {
   float c1, c2z, c2x, e, damp, dlen;
 };
+template <bool ARD = false>
 __device__ __forceinline__ FactorAdj factor_adjoint(int type, const float* x, const float* z, int d, float amp,
-                                                    float len, float nx, float nz, float kval, float gk) {
+                                                    float len, float nx, float nz, float kval, float gk,
+                                                    const float* il = nullptr) {
   FactorAdj a = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   if (type == SVGP_K_SE) {
     float r2 = 0.f;
-    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; r2 = fmaf(t, t, r2); }
+    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; if (ARD) t *= il[f]; r2 = fmaf(t, t, r2); }
     float il2 = 1.0f / (len * len);
     a.c1 = gk * kval * il2;      // dk/dz_f = k (x_f - z_f)/l^2
     a.c2z = -a.c1;
@@ -164,7 +175,7 @@ __device__ __forceinline__ FactorAdj factor_adjoint(int type, const float* x, co
     // for nu = 3/2, 5/2 and no division by r appears.  nu = 1/2 has C = k / (l r): 0 at r = 0 (the symmetric subgradient,
     // which gives the exact total derivative of k(z, z) = a^2 when both sides are summed, as the K_mm adjoint does)
     float r2 = 0.f;
-    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; r2 = fmaf(t, t, r2); }
+    for (int f = 0; f < d; ++f) { float t = x[f] - z[f]; if (ARD) t *= il[f]; r2 = fmaf(t, t, r2); }
     const float r = sqrtf(r2), u = matern_c(type) * r / len;
     const float il2 = 1.0f / (len * len);
     float C, dl;
@@ -219,6 +230,33 @@ __device__ __forceinline__ void load_features(const float* F, int64_t ld, int64_
 }
 
 // ------------------------------------------------------------------------------------------
+// ARD (SVGP_K_ARD): one length scale l_f per feature column of a block, at hyp[4 + f].  The ARD instantiations of the
+// generic kernels keep the inverse length scales in ARD_SMEM bytes behind their own shared-memory layout (float il[MAXD]
+// for the fp32 passes, double il[MAXD] for the float64 evaluations) and evaluate an ARD factor with len = 1; the
+// features of an isotropic block get il = 1 (exact), so its factor keeps its own len.  Every kernel without ARD is
+// the same code as without the flag.
+// ------------------------------------------------------------------------------------------
+constexpr size_t ARD_SMEM = MAXD * (sizeof(float) + sizeof(double));
+__device__ __forceinline__ bool ard_feature(Spec sp, int f) { return f < sp.da ? sp.ard_a : sp.ard_b; }
+// written by the first d threads: callers synchronise before the first read (load_features does)
+__device__ __forceinline__ void load_ard(const float* hyp, Spec sp, float* ilf, double* ild) {
+  for (int f = threadIdx.x; f < sp.da + sp.db; f += blockDim.x) {
+    const double il = ard_feature(sp, f) ? 1.0 / (double)hyp[4 + f] : 1.0;
+    if (ilf) ilf[f] = (float)il;
+    if (ild) ild[f] = il;
+  }
+}
+__device__ __forceinline__ Hyp ard_hyp(Hyp h, Spec sp) {
+  if (sp.ard_a) h.len_a = 1.f;
+  if (sp.ard_b) h.len_b = 1.f;
+  return h;
+}
+// length scale of feature f (SE44 kernels: the eight of them live in registers)
+__device__ __forceinline__ float ard_len(const float* hyp, Spec sp, Hyp h, int f) {
+  return ard_feature(sp, f) ? hyp[4 + f] : (f < sp.da ? h.len_a : h.len_b);
+}
+
+// ------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------
 // Power-of-two scale of the fp16 planes: the kernel's upper bound (amplitude^2 for the stationary factors,
@@ -266,6 +304,7 @@ __global__ void feature_norm_kernel(const float* __restrict__ F, int64_t ld, int
   }
 }
 
+template <bool ARD = false>
 __global__ void __launch_bounds__(THREADS) kernel_fwd_kernel(
     const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz, int64_t M,
     Spec sp, const float* __restrict__ hyp, float* __restrict__ K, int64_t ldk, __half* __restrict__ Kh,
@@ -280,7 +319,9 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_kernel(
   float* nxb = nxa + TILE;
   float* nza = nxb + TILE;
   float* nzb = nza + TILE;
-  const Hyp h = load_hyp(hyp);
+  float* il = nzb + TILE;              // ARD: [MAXD]
+  const Hyp h = ARD ? ard_hyp(load_hyp(hyp), sp) : load_hyp(hyp);
+  if (ARD) load_ard(hyp, sp, il, nullptr);
   const int64_t col0 = (int64_t)blockIdx.x * TILE;
   const int64_t ntiles_r = (N + TILE - 1) / TILE;
   float scale = 1.0f;
@@ -299,8 +340,9 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_kernel(
 #pragma unroll 4
     for (int j = 0; j < TILE / 4; ++j) {
       int r = rg + 4 * j;
-      float ka = factor_value(sp.ta, xs + r * dp, zs + c * dp, sp.da, h.amp_a, h.len_a, nxa[r], nza[c]);
-      float kb = factor_value(sp.tb, xs + r * dp + sp.da, zs + c * dp + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c]);
+      float ka = factor_value<ARD>(sp.ta, xs + r * dp, zs + c * dp, sp.da, h.amp_a, h.len_a, nxa[r], nza[c], il);
+      float kb = factor_value<ARD>(sp.tb, xs + r * dp + sp.da, zs + c * dp + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c],
+                                   il + sp.da);
       tile[r * (TILE + 1) + c] = ka * kb;
     }
     __syncthreads();
@@ -349,8 +391,8 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_kernel(
 // packed {hi, lo} words (pitch 65: conflict-free for the column-per-lane writes and for both read-outs below) and
 // every thread leaves with 16-byte stores -- 8 consecutive columns of a row of Kh / Kl, 8 consecutive datapoints of
 // a row of Kth / Ktl.  SE44 = product of two 4-feature SE factors (the SWEEP kernel): inducing features live in
-// registers, datapoint features are broadcast float4 loads, both factors share one ex2.
-template <bool SE44>
+// registers, datapoint features are broadcast float4 loads, both factors share one ex2.  ARD specs take the generic form.
+template <bool SE44, bool ARD = false>
 __global__ void __launch_bounds__(THREADS) kernel_fwd_planes_kernel(
     const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz, int64_t M,
     Spec sp, const float* __restrict__ hyp, __half* __restrict__ Kh, __half* __restrict__ Kl, int64_t ldkh,
@@ -365,8 +407,11 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_planes_kernel(
   float* nxb = nxa + TILE;
   float* nza = nxb + TILE;
   float* nzb = nza + TILE;
+  float* il = nzb + TILE;                             // ARD: [MAXD]
   constexpr int P = TILE + 1;
-  const Hyp h = load_hyp(hyp);
+  static_assert(!(SE44 && ARD), "ARD specs take the generic planes builder");
+  const Hyp h = ARD ? ard_hyp(load_hyp(hyp), sp) : load_hyp(hyp);
+  if (ARD) load_ard(hyp, sp, il, nullptr);
   const int64_t col0 = (int64_t)blockIdx.x * TILE;
   const int64_t ntiles_r = (N + TILE - 1) / TILE;
   const float scale = plane_scale(sp, h, kscale);
@@ -412,8 +457,9 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_planes_kernel(
         t = xb.w - zr[7]; rb = fmaf(t, t, rb);
         vs = amp2s * exp2f(fmaf(ca, ra, cb * rb));
       } else {
-        const float ka = factor_value(sp.ta, xs + r * dpx, zs + c * dpz, sp.da, h.amp_a, h.len_a, nxa[r], nza[c]);
-        const float kb = factor_value(sp.tb, xs + r * dpx + sp.da, zs + c * dpz + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c]);
+        const float ka = factor_value<ARD>(sp.ta, xs + r * dpx, zs + c * dpz, sp.da, h.amp_a, h.len_a, nxa[r], nza[c], il);
+        const float kb = factor_value<ARD>(sp.tb, xs + r * dpx + sp.da, zs + c * dpz + sp.da, sp.db, h.amp_b, h.len_b, nxb[r],
+                                           nzb[c], il + sp.da);
         vs = ka * kb * scale;
       }
       if (row0 + r >= N) vs = 0.f;                    // datapoints past N are zero in the blocked transpose
@@ -474,20 +520,26 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_planes_kernel(
 // float64 kernel matrix (fp32 features, float64 arithmetic): OutT = double is K_mm of the M x M stage; OutT = float is the plain
 // K_nm of the small (SIMT-path) problems, ONE rounding of the float64 value -- the fp32 evaluation of the exponential carries
 // ~5e-7 of relative error (rounding of its argument), which e.g. the (b x b) solve of the Titsias bound amplifies to 1.2e-4 in dy
-template <typename OutT>
+// ARD: launched with MAXD doubles of dynamic shared memory for the inverse length scales
+template <typename OutT, bool ARD = false>
 __global__ void kernel_fwd_f64_kernel(const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz,
                                       int64_t M, Spec sp, const float* __restrict__ hyp, OutT* __restrict__ K, int64_t ldk) {
-  const Hyp h = load_hyp(hyp);
+  extern __shared__ double il_f64[];
+  const Hyp h = ARD ? ard_hyp(load_hyp(hyp), sp) : load_hyp(hyp);
+  if (ARD) {
+    load_ard(hyp, sp, nullptr, il_f64);
+    __syncthreads();
+  }
   const int64_t total = N * M;
   for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
     const int64_t i = idx / M, j = idx - i * M;
     const float* x = Fx + i * ldx;
     const float* z = Fz + j * ldz;
-    const double ka = factor_value_f64(sp.ta, x, z, sp.da, h.amp_a, h.len_a, sp.ta == SVGP_K_COSINE ? block_norm_f64(x, sp.da) : 1.0,
-                                       sp.ta == SVGP_K_COSINE ? block_norm_f64(z, sp.da) : 1.0);
-    const double kb = factor_value_f64(sp.tb, x + sp.da, z + sp.da, sp.db, h.amp_b, h.len_b,
-                                       sp.tb == SVGP_K_COSINE ? block_norm_f64(x + sp.da, sp.db) : 1.0,
-                                       sp.tb == SVGP_K_COSINE ? block_norm_f64(z + sp.da, sp.db) : 1.0);
+    const double ka = factor_value_f64<ARD>(sp.ta, x, z, sp.da, h.amp_a, h.len_a, sp.ta == SVGP_K_COSINE ? block_norm_f64(x, sp.da) : 1.0,
+                                            sp.ta == SVGP_K_COSINE ? block_norm_f64(z, sp.da) : 1.0, il_f64);
+    const double kb = factor_value_f64<ARD>(sp.tb, x + sp.da, z + sp.da, sp.db, h.amp_b, h.len_b,
+                                            sp.tb == SVGP_K_COSINE ? block_norm_f64(x + sp.da, sp.db) : 1.0,
+                                            sp.tb == SVGP_K_COSINE ? block_norm_f64(z + sp.da, sp.db) : 1.0, il_f64 + sp.da);
     K[i * ldk + j] = (OutT)(ka * kb);
   }
 }
@@ -499,7 +551,9 @@ __global__ void kernel_fwd_f64_kernel(const float* __restrict__ Fx, int64_t ldx,
 // would stop at 22 bits; the M = 2048 sweep point needs more: tools/numerics/sim_parity.py) -- plus the fp16 hi/lo row
 // planes the remaining fp16 consumers read.  Two passes over the same tiles: MAXPASS = true only reduces the row and
 // column maxima (float bits, atomicMax), MAXPASS = false writes.
-template <bool SE44, bool MAXPASS>
+// ARD: the generic form reads the inverse length scales from shared memory (ARD_SMEM behind the layout); SE44 keeps the
+// per-feature exponent factors -log2(e) / (2 l_f^2) in registers, in fp32 for the maxima and in float64 for the write
+template <bool SE44, bool MAXPASS, bool ARD = false>
 __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
     const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz, int64_t M,
     Spec sp, const float* __restrict__ hyp, __half* __restrict__ Kh, __half* __restrict__ Kl, int64_t ldkh,
@@ -515,6 +569,8 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
   float* nxb = nxa + TILE;
   float* nza = nxb + TILE;
   float* nzb = nza + TILE;
+  float* il = nzb + TILE;                             // ARD, generic: float[MAXD], then double[MAXD]
+  double* ild = reinterpret_cast<double*>(il + MAXD);
   constexpr int P = TILE + 1;
   // POWER-OF-TWO fixed-point grids: max = m 2^e (m in [0.5, 1)) -> integer = value * 2^(31 - e) (2^(30 - e) when m > 0.99).  The
   // product with a power of two is exact in fp32 and a 24-bit mantissa within 2^-7 of the maximum fits the grid whole, so
@@ -529,7 +585,8 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
     e = e > 120 ? 120 : (e < -120 ? -120 : e);
     return ldexpf(1.0f, e);
   };
-  const Hyp h = load_hyp(hyp);
+  const Hyp h = ARD ? ard_hyp(load_hyp(hyp), sp) : load_hyp(hyp);
+  if (ARD && !SE44) load_ard(hyp, sp, il, ild);
   const int64_t col0 = (int64_t)blockIdx.x * TILE;
   const int64_t ntiles_r = (N + TILE - 1) / TILE;
   const float scale = plane_scale(sp, h, kscale);
@@ -542,6 +599,8 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
   const int k4 = lane & 3, sub = lane >> 2;
   float zr[8];
   float ca = 0.f, cb = 0.f, amp2 = 0.f;
+  float cf[ARD ? 8 : 1];                              // SE44 + ARD: -log2(e) / (2 l_f^2), fp32 (maxima) ...
+  double cfd[ARD ? 8 : 1];                            // ... and float64 (write pass)
   if (SE44) {
 #pragma unroll
     for (int f = 0; f < 8; ++f) zr[f] = zs[c * dpz + f];
@@ -549,6 +608,14 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
     ca = -0.5f * LOG2E / (h.len_a * h.len_a);
     cb = -0.5f * LOG2E / (h.len_b * h.len_b);
     amp2 = h.amp_a * h.amp_a * h.amp_b * h.amp_b;
+    if (ARD) {
+#pragma unroll
+      for (int f = 0; f < 8; ++f) {
+        const double l = ard_len(hyp, sp, h, f);
+        if (MAXPASS) cf[f] = -0.5f * LOG2E / (float)(l * l);
+        else cfd[f] = -0.5 * 1.4426950408889634 / (l * l);
+      }
+    }
   }
   const double LOG2E_D = 1.4426950408889634;
   const double cad = -0.5 * LOG2E_D / ((double)h.len_a * (double)h.len_a), cbd = -0.5 * LOG2E_D / ((double)h.len_b * (double)h.len_b);
@@ -571,7 +638,24 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
     for (int j = 0; j < TILE / 4; ++j) {
       const int r = rg + 4 * j;
       float v;
-      if (SE44 && MAXPASS) {
+      if (SE44 && ARD) {
+        // exponent sum_f c_f (x_f - z_f)^2: fp32 for the maxima; for the write pass the float64 difference times the
+        // float64 c_f (one DMUL per feature on top of the isotropic form) and one rounding at the end
+        const float4 xa = *reinterpret_cast<const float4*>(xs + r * 8);
+        const float4 xb = *reinterpret_cast<const float4*>(xs + r * 8 + 4);
+        const float xv[8] = {xa.x, xa.y, xa.z, xa.w, xb.x, xb.y, xb.z, xb.w};
+        if (MAXPASS) {
+          float e = 0.f;
+#pragma unroll
+          for (int f = 0; f < 8; ++f) { const float t = xv[f] - zr[f]; e = fmaf(cf[f] * t, t, e); }
+          v = amp2 * exp2f(e);
+        } else {
+          double e = 0.0;
+#pragma unroll
+          for (int f = 0; f < 8; ++f) { const double t = (double)xv[f] - (double)zr[f]; e = fma(cfd[f] * t, t, e); }
+          v = (float)(amp2d * exp2(e));
+        }
+      } else if (SE44 && MAXPASS) {
         const float4 xa = *reinterpret_cast<const float4*>(xs + r * 8);
         const float4 xb = *reinterpret_cast<const float4*>(xs + r * 8 + 4);
         float t, ra, rb;
@@ -599,16 +683,18 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
         t = (double)xb.w - (double)zr[7]; rb = fma(t, t, rb);
         v = (float)(amp2d * exp2(fma(cad, ra, cbd * rb)));
       } else if (MAXPASS) {
-        const float ka = factor_value(sp.ta, xs + r * dpx, zs + c * dpz, sp.da, h.amp_a, h.len_a, nxa[r], nza[c]);
-        const float kb = factor_value(sp.tb, xs + r * dpx + sp.da, zs + c * dpz + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c]);
+        const float ka = factor_value<ARD>(sp.ta, xs + r * dpx, zs + c * dpz, sp.da, h.amp_a, h.len_a, nxa[r], nza[c], il);
+        const float kb = factor_value<ARD>(sp.tb, xs + r * dpx + sp.da, zs + c * dpz + sp.da, sp.db, h.amp_b, h.len_b, nxb[r],
+                                           nzb[c], il + sp.da);
         v = ka * kb;
       } else {
-        const double ka = factor_value_f64(sp.ta, xs + r * dpx, zs + c * dpz, sp.da, h.amp_a, h.len_a,
-                                           sp.ta == SVGP_K_COSINE ? block_norm_f64(xs + r * dpx, sp.da) : 1.0,
-                                           sp.ta == SVGP_K_COSINE ? block_norm_f64(zs + c * dpz, sp.da) : 1.0);
-        const double kb = factor_value_f64(sp.tb, xs + r * dpx + sp.da, zs + c * dpz + sp.da, sp.db, h.amp_b, h.len_b,
-                                           sp.tb == SVGP_K_COSINE ? block_norm_f64(xs + r * dpx + sp.da, sp.db) : 1.0,
-                                           sp.tb == SVGP_K_COSINE ? block_norm_f64(zs + c * dpz + sp.da, sp.db) : 1.0);
+        const double ka = factor_value_f64<ARD>(sp.ta, xs + r * dpx, zs + c * dpz, sp.da, h.amp_a, h.len_a,
+                                                sp.ta == SVGP_K_COSINE ? block_norm_f64(xs + r * dpx, sp.da) : 1.0,
+                                                sp.ta == SVGP_K_COSINE ? block_norm_f64(zs + c * dpz, sp.da) : 1.0, ild);
+        const double kb = factor_value_f64<ARD>(sp.tb, xs + r * dpx + sp.da, zs + c * dpz + sp.da, sp.db, h.amp_b, h.len_b,
+                                                sp.tb == SVGP_K_COSINE ? block_norm_f64(xs + r * dpx + sp.da, sp.db) : 1.0,
+                                                sp.tb == SVGP_K_COSINE ? block_norm_f64(zs + c * dpz + sp.da, sp.db) : 1.0,
+                                                ild + sp.da);
         v = (float)(ka * kb);
       }
       if (row0 + r >= N || col0 + c >= M) v = 0.f;
@@ -714,8 +800,12 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
 //           one flush per block)
 // ACC64 (pass Z of the Matern factors): the per-tile fp32 partials are folded into double across the row tiles and the
 // flush  dz_f = sum c1 x_f + z_f sum c2z  (which cancels: c2z = -c1) is done in double, as in kernel_bwd_z_se44_kernel
+// ARD: the coefficients are those of the scaled coordinates (factor_adjoint), the phase-2 sums run on the unscaled
+// features, and the flush multiplies by il_f^2.  Pass Z also sums  c1 (x_f - z_f)^2  per entry for every feature of an
+// ARD block (fp32 per tile, folded into double): dl_f = il_f^3 times that.  (Per-column moments sum c1 x^2, sum c1 x,
+// sum c1 would cancel by orders of magnitude in fp32 for offset features such as time stamps.)
 // ------------------------------------------------------------------------------------------
-template <bool PASS_X, bool ACC64 = false>
+template <bool PASS_X, bool ACC64 = false, bool ARD = false>
 __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
     const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz, int64_t M,
     Spec sp, const float* __restrict__ hyp, const float* __restrict__ G, int64_t ldg, float* __restrict__ dFx,
@@ -733,7 +823,9 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
   float* nzb = nza + TILE;
   float* own = nzb + TILE;                      // [TILE][4]: scalar coefficients on own features {c2 A, c2 B, e A, e B}
   float* hred = own + TILE * 4;                 // [4] hyper partials (float atomics in smem)
-  const Hyp h = load_hyp(hyp);
+  float* il = hred + 4;                         // ARD: [MAXD]
+  const Hyp h = ARD ? ard_hyp(load_hyp(hyp), sp) : load_hyp(hyp);
+  if (ARD) load_ard(hyp, sp, il, nullptr);
   const int c = threadIdx.x % TILE, rg = threadIdx.x / TILE;
   const int64_t ntr = (N + TILE - 1) / TILE, ntc = (M + TILE - 1) / TILE;
 
@@ -751,6 +843,9 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
     for (int q = 0; q < (ACC64 ? MAXD / 4 : 1); ++q) acc64[q] = 0.0;
     // hyper-parameter gradients are heavily cancelling sums over all N x M entries: accumulate them in double
     double hy[4] = {0.0, 0.0, 0.0, 0.0};
+    double hyl[ARD && !PASS_X ? MAXD / 4 : 1];   // ARD: sum c1 (x_f - z_f)^2 of the owned column, features fg + 4q
+#pragma unroll
+    for (int q = 0; q < (ARD && !PASS_X ? MAXD / 4 : 1); ++q) hyl[q] = 0.0;
     if (threadIdx.x < 4) hred[threadIdx.x] = 0.f;
     if (PASS_X) load_features(Fx, ldx, ot * TILE, N, d, dp, sp, xs, nxa, nxb);
     else        load_features(Fz, ldz, ot * TILE, M, d, dp, sp, zs, nza, nzb);
@@ -769,10 +864,13 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
         float g = (gr < N && gc < M) ? G[gr * ldg + gc] : 0.f;
         const float* xa = xs + r * dp;
         const float* za = zs + c * dp;
-        float ka = factor_value(sp.ta, xa, za, sp.da, h.amp_a, h.len_a, nxa[r], nza[c]);
-        float kb = factor_value(sp.tb, xa + sp.da, za + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c]);
-        FactorAdj A = factor_adjoint(sp.ta, xa, za, sp.da, h.amp_a, h.len_a, nxa[r], nza[c], ka, g * kb);
-        FactorAdj B = factor_adjoint(sp.tb, xa + sp.da, za + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c], kb, g * ka);
+        float ka = factor_value<ARD>(sp.ta, xa, za, sp.da, h.amp_a, h.len_a, nxa[r], nza[c], il);
+        float kb = factor_value<ARD>(sp.tb, xa + sp.da, za + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c], il + sp.da);
+        FactorAdj A = factor_adjoint<ARD>(sp.ta, xa, za, sp.da, h.amp_a, h.len_a, nxa[r], nza[c], ka, g * kb, il);
+        FactorAdj B = factor_adjoint<ARD>(sp.tb, xa + sp.da, za + sp.da, sp.db, h.amp_b, h.len_b, nxb[r], nzb[c], kb, g * ka,
+                                          il + sp.da);
+        if (ARD && sp.ard_a) A.dlen = 0.f;        // an ARD block's isotropic slot gets exactly 0
+        if (ARD && sp.ard_b) B.dlen = 0.f;
         c1a[r * (TILE + 1) + c] = A.c1;
         c1b[r * (TILE + 1) + c] = B.c1;
         if (PASS_X) {
@@ -808,6 +906,15 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
             }
             if (ACC64) acc64[q] += (double)s;
             else acc[q] += s;
+            if (ARD && !PASS_X && ard_feature(sp, f)) {
+              const float zf = zs[o * dp + f];
+              float s2 = 0.f;
+              for (int k = 0; k < TILE; ++k) {
+                const float t = xs[k * dp + f] - zf;
+                s2 = fmaf(cmat[k * (TILE + 1) + o] * t, t, s2);
+              }
+              hyl[q] += (double)s2;
+            }
           }
         }
         if (ACC64) {          // every thread keeps its own copy: the flush needs no broadcast
@@ -837,6 +944,7 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
           double v = acc64[q] + own64[inA ? 0 : 1] * (double)self[f];
           if (inA && f == 0 && sp.ta == SVGP_K_EXPSIN) v += own64[2];
           if (!inA && f == sp.da && sp.tb == SVGP_K_EXPSIN) v += own64[3];
+          if (ARD) v *= (double)il[f] * (double)il[f];
           if (go < M) atomicAdd(&dFz[go * d + f], v);
           continue;
         }
@@ -844,6 +952,7 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
         // EXPSIN contributes only through its single feature (the first of its block)
         if (inA && f == 0 && sp.ta == SVGP_K_EXPSIN) v += own[o * 4 + 2];
         if (!inA && f == sp.da && sp.tb == SVGP_K_EXPSIN) v += own[o * 4 + 3];
+        if (ARD) v *= il[f] * il[f];
         if (PASS_X) {
           if (go < N) dFx[go * d + f] = v;
         } else {
@@ -858,6 +967,19 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
           for (int o2 = 16; o2 > 0; o2 >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o2);
           if ((threadIdx.x & 31) == 0) atomicAdd(&dhyp[k], s);          // one double atomic per warp per owned tile
         }
+        if (ARD) {
+          // the 32 lanes of a warp share fg: one double atomic per warp and ARD feature
+#pragma unroll
+          for (int q = 0; q < MAXD / 4; ++q) {
+            const int f = fg + 4 * q;
+            if (f >= d || !ard_feature(sp, f)) continue;
+            const double l = hyp[4 + f];
+            double s = hyl[q] / (l * l * l);
+#pragma unroll
+            for (int o2 = 16; o2 > 0; o2 >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o2);
+            if ((threadIdx.x & 31) == 0) atomicAdd(&dhyp[4 + f], s);
+          }
+        }
       }
       __syncthreads();
     }
@@ -870,12 +992,17 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
 // a thread owns one inducing point (features in registers) and 16 of the 64 datapoints of a tile, the datapoint
 // features are broadcast float4 loads, g is read in coalesced 128-byte rows; one float partial per tile, folded into
 // double per thread (the hyper-parameter sums cancel heavily), one double atomic per (column, feature) per block.
+// ARD (either block): the exponent is sum_f c_f d_f^2 with c_f = -log2(e) / (2 l_f^2), and the eight per-feature sums
+// sum c d_f^2 take the place of the two per-block sums sum c r2 (17 partials instead of 11); dz_f = (...) / l_f^2,
+// dl_f = sum c d_f^2 / l_f^3, and an isotropic block's dl is the sum of its four.
+template <bool ARD = false>
 __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
     const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz, int64_t M,
     const float* __restrict__ hyp, const float* __restrict__ G, int64_t ldg, double* __restrict__ dFz,
-    double* __restrict__ dhyp) {
+    double* __restrict__ dhyp, Spec sp) {
+  constexpr int NS = ARD ? 17 : 11, NH = ARD ? 12 : 4;   // partials per thread, dhyp slots
   __shared__ __align__(16) float xs[TILE * 8];
-  __shared__ double red[4][TILE][11];            // per row group: 8 feature sums, sum c, sum c r2a, sum c r2b
+  __shared__ double red[4][TILE][NS];            // per row group: 8 feature sums, sum c, sum c r2a, sum c r2b (ARD: 8 x sum c d_f^2)
   const Hyp h = load_hyp(hyp);
   const int c = threadIdx.x % TILE, rg = threadIdx.x / TILE;
   const int64_t ntr = (N + TILE - 1) / TILE;
@@ -886,9 +1013,14 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
   const float LOG2E = 1.4426950408889634f;
   const float ca = -0.5f * LOG2E / (h.len_a * h.len_a), cb = -0.5f * LOG2E / (h.len_b * h.len_b);
   const float amp2 = h.amp_a * h.amp_a * h.amp_b * h.amp_b;
-  double acc[11];
+  float cf[ARD ? 8 : 1];
+  if (ARD) {
 #pragma unroll
-  for (int q = 0; q < 11; ++q) acc[q] = 0.0;
+    for (int f = 0; f < 8; ++f) { const float l = ard_len(hyp, sp, h, f); cf[f] = -0.5f * LOG2E / (l * l); }
+  }
+  double acc[NS];
+#pragma unroll
+  for (int q = 0; q < NS; ++q) acc[q] = 0.0;
   for (int64_t rt = blockIdx.y; rt < ntr; rt += gridDim.y) {
     const int64_t row0 = rt * TILE;
     __syncthreads();
@@ -897,9 +1029,9 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
       xs[idx] = gr < N ? Fx[gr * ldx + (idx & 7)] : 0.f;
     }
     __syncthreads();
-    float t[11];
+    float t[NS];
 #pragma unroll
-    for (int q = 0; q < 11; ++q) t[q] = 0.f;
+    for (int q = 0; q < NS; ++q) t[q] = 0.f;
 #pragma unroll 4
     for (int j = 0; j < TILE / 4; ++j) {
       const int r = rg + 4 * j;
@@ -909,6 +1041,19 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
       const float4 xb = *reinterpret_cast<const float4*>(xs + r * 8 + 4);
       float d0 = xa.x - z[0], d1 = xa.y - z[1], d2 = xa.z - z[2], d3 = xa.w - z[3];
       float e0 = xb.x - z[4], e1 = xb.y - z[5], e2 = xb.z - z[6], e3 = xb.w - z[7];
+      if (ARD) {
+        const float sq[8] = {d0 * d0, d1 * d1, d2 * d2, d3 * d3, e0 * e0, e1 * e1, e2 * e2, e3 * e3};
+        float ex = 0.f;
+#pragma unroll
+        for (int f = 0; f < 8; ++f) ex = fmaf(cf[f], sq[f], ex);
+        const float ck = g * amp2 * exp2f(ex);
+        t[0] = fmaf(ck, xa.x, t[0]); t[1] = fmaf(ck, xa.y, t[1]); t[2] = fmaf(ck, xa.z, t[2]); t[3] = fmaf(ck, xa.w, t[3]);
+        t[4] = fmaf(ck, xb.x, t[4]); t[5] = fmaf(ck, xb.y, t[5]); t[6] = fmaf(ck, xb.z, t[6]); t[7] = fmaf(ck, xb.w, t[7]);
+        t[8] += ck;
+#pragma unroll
+        for (int f = 0; f < 8; ++f) t[9 + f] = fmaf(ck, sq[f], t[9 + f]);
+        continue;
+      }
       const float ra = fmaf(d3, d3, fmaf(d2, d2, fmaf(d1, d1, d0 * d0)));
       const float rb = fmaf(e3, e3, fmaf(e2, e2, fmaf(e1, e1, e0 * e0)));
       const float ck = g * amp2 * exp2f(fmaf(ca, ra, cb * rb));
@@ -917,15 +1062,32 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
       t[8] += ck; t[9] = fmaf(ck, ra, t[9]); t[10] = fmaf(ck, rb, t[10]);
     }
 #pragma unroll
-    for (int q = 0; q < 11; ++q) acc[q] += (double)t[q];
+    for (int q = 0; q < NS; ++q) acc[q] += (double)t[q];
   }
 #pragma unroll
-  for (int q = 0; q < 11; ++q) red[rg][c][q] = acc[q];
+  for (int q = 0; q < NS; ++q) red[rg][c][q] = acc[q];
   __syncthreads();
-  if (rg == 0 && gc < M) {
-    double s[11];
+  if (ARD && rg == 0 && gc < M) {
+    double s[NS], dl[8];
 #pragma unroll
-    for (int q = 0; q < 11; ++q) s[q] = red[0][c][q] + red[1][c][q] + red[2][c][q] + red[3][c][q];
+    for (int q = 0; q < NS; ++q) s[q] = red[0][c][q] + red[1][c][q] + red[2][c][q] + red[3][c][q];
+#pragma unroll
+    for (int f = 0; f < 8; ++f) {
+      const double l = ard_len(hyp, sp, h, f), il2 = 1.0 / (l * l);
+      atomicAdd(&dFz[gc * 8 + f], (s[f] - (double)z[f] * s[8]) * il2);
+      dl[f] = s[9 + f] * il2 / l;
+    }
+    red[0][c][0] = 2.0 * s[8] / h.amp_a; red[0][c][1] = sp.ard_a ? 0.0 : dl[0] + dl[1] + dl[2] + dl[3];
+    red[0][c][2] = 2.0 * s[8] / h.amp_b; red[0][c][3] = sp.ard_b ? 0.0 : dl[4] + dl[5] + dl[6] + dl[7];
+#pragma unroll
+    for (int f = 0; f < 8; ++f) red[0][c][4 + f] = ard_feature(sp, f) ? dl[f] : 0.0;
+  } else if (ARD && rg == 0) {
+#pragma unroll
+    for (int k = 0; k < NH; ++k) red[0][c][k] = 0.0;
+  } else if (rg == 0 && gc < M) {
+    double s[NS];
+#pragma unroll
+    for (int q = 0; q < NS; ++q) s[q] = red[0][c][q] + red[1][c][q] + red[2][c][q] + red[3][c][q];
     const double ila = 1.0 / ((double)h.len_a * h.len_a), ilb = 1.0 / ((double)h.len_b * h.len_b);
 #pragma unroll
     for (int f = 0; f < 8; ++f) atomicAdd(&dFz[gc * 8 + f], (s[f] - (double)z[f] * s[8]) * (f < 4 ? ila : ilb));
@@ -935,7 +1097,7 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
     red[0][c][0] = red[0][c][1] = red[0][c][2] = red[0][c][3] = 0.0;
   }
   __syncthreads();
-  if (threadIdx.x < 4) {
+  if (threadIdx.x < NH) {
     double s = 0.0;
     for (int k = 0; k < TILE; ++k) s += red[0][k][threadIdx.x];
     atomicAdd(&dhyp[threadIdx.x], s);
@@ -945,10 +1107,18 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
 // ------------------------------------------------------------------------------------------
 // element-wise apply (diag_only=True)
 // ------------------------------------------------------------------------------------------
+// ARD: launched with ARD_SMEM bytes of dynamic shared memory (the inverse length scales; the adjoint also keeps its
+// per-feature dl_f partials there)
+template <bool ARD = false>
 __global__ void kernel_diag_fwd_kernel(const float* __restrict__ Fx, int64_t ldx, const float* __restrict__ Fy,
                                        int64_t ldy, int64_t N, Spec sp, const float* __restrict__ hyp,
                                        float* __restrict__ kd) {
-  const Hyp h = load_hyp(hyp);
+  extern __shared__ float il_diag[];
+  const Hyp h = ARD ? ard_hyp(load_hyp(hyp), sp) : load_hyp(hyp);
+  if (ARD) {
+    load_ard(hyp, sp, il_diag, nullptr);
+    __syncthreads();
+  }
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
     float x[MAXD], y[MAXD];
     const int d = sp.da + sp.db;
@@ -956,17 +1126,25 @@ __global__ void kernel_diag_fwd_kernel(const float* __restrict__ Fx, int64_t ldx
     float nxa = 1.f, nya = 1.f, nxb = 1.f, nyb = 1.f;
     if (sp.ta == SVGP_K_COSINE) { nxa = block_norm(x, sp.da); nya = block_norm(y, sp.da); }
     if (sp.tb == SVGP_K_COSINE) { nxb = block_norm(x + sp.da, sp.db); nyb = block_norm(y + sp.da, sp.db); }
-    float ka = factor_value(sp.ta, x, y, sp.da, h.amp_a, h.len_a, nxa, nya);
-    float kb = factor_value(sp.tb, x + sp.da, y + sp.da, sp.db, h.amp_b, h.len_b, nxb, nyb);
+    float ka = factor_value<ARD>(sp.ta, x, y, sp.da, h.amp_a, h.len_a, nxa, nya, il_diag);
+    float kb = factor_value<ARD>(sp.tb, x + sp.da, y + sp.da, sp.db, h.amp_b, h.len_b, nxb, nyb, il_diag + sp.da);
     kd[i] = ka * kb;
   }
 }
 
+template <bool ARD = false>
 __global__ void kernel_diag_bwd_kernel(const float* __restrict__ Fx, int64_t ldx, const float* __restrict__ Fy,
                                        int64_t ldy, int64_t N, Spec sp, const float* __restrict__ hyp,
                                        const float* __restrict__ g, float* __restrict__ dFx, float* __restrict__ dFy,
                                        double* __restrict__ dhyp) {
-  const Hyp h = load_hyp(hyp);
+  extern __shared__ float il_diag[];
+  double* dl = reinterpret_cast<double*>(il_diag + MAXD);       // ARD: this block's sum c1 (x_f - y_f)^2 il_f^3
+  const Hyp h = ARD ? ard_hyp(load_hyp(hyp), sp) : load_hyp(hyp);
+  if (ARD) {
+    load_ard(hyp, sp, il_diag, nullptr);
+    for (int f = threadIdx.x; f < MAXD; f += blockDim.x) dl[f] = 0.0;
+    __syncthreads();
+  }
   double hy[4] = {0.0, 0.0, 0.0, 0.0};
   const int d = sp.da + sp.db;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
@@ -975,16 +1153,27 @@ __global__ void kernel_diag_bwd_kernel(const float* __restrict__ Fx, int64_t ldx
     float nxa = 1.f, nya = 1.f, nxb = 1.f, nyb = 1.f;
     if (sp.ta == SVGP_K_COSINE) { nxa = block_norm(x, sp.da); nya = block_norm(y, sp.da); }
     if (sp.tb == SVGP_K_COSINE) { nxb = block_norm(x + sp.da, sp.db); nyb = block_norm(y + sp.da, sp.db); }
-    float ka = factor_value(sp.ta, x, y, sp.da, h.amp_a, h.len_a, nxa, nya);
-    float kb = factor_value(sp.tb, x + sp.da, y + sp.da, sp.db, h.amp_b, h.len_b, nxb, nyb);
+    float ka = factor_value<ARD>(sp.ta, x, y, sp.da, h.amp_a, h.len_a, nxa, nya, il_diag);
+    float kb = factor_value<ARD>(sp.tb, x + sp.da, y + sp.da, sp.db, h.amp_b, h.len_b, nxb, nyb, il_diag + sp.da);
     float gi = g[i];
-    FactorAdj A = factor_adjoint(sp.ta, x, y, sp.da, h.amp_a, h.len_a, nxa, nya, ka, gi * kb);
-    FactorAdj B = factor_adjoint(sp.tb, x + sp.da, y + sp.da, sp.db, h.amp_b, h.len_b, nxb, nyb, kb, gi * ka);
+    FactorAdj A = factor_adjoint<ARD>(sp.ta, x, y, sp.da, h.amp_a, h.len_a, nxa, nya, ka, gi * kb, il_diag);
+    FactorAdj B = factor_adjoint<ARD>(sp.tb, x + sp.da, y + sp.da, sp.db, h.amp_b, h.len_b, nxb, nyb, kb, gi * ka,
+                                      il_diag + sp.da);
+    if (ARD && sp.ard_a) A.dlen = 0.f;
+    if (ARD && sp.ard_b) B.dlen = 0.f;
     for (int f = 0; f < d; ++f) {
       const FactorAdj& T = (f < sp.da) ? A : B;
       int type = (f < sp.da) ? sp.ta : sp.tb;
       bool first = (f == 0) || (f == sp.da);
       float ex = (type == SVGP_K_EXPSIN && first) ? T.e : 0.f;
+      if (ARD) {
+        const float il2 = il_diag[f] * il_diag[f];
+        dFx[i * d + f] = (T.c1 * y[f] + T.c2x * x[f] - ex) * il2;
+        dFy[i * d + f] = (T.c1 * x[f] + T.c2z * y[f] + ex) * il2;
+        const float t = x[f] - y[f];
+        if (ard_feature(sp, f) && T.c1 * t != 0.f) atomicAdd(&dl[f], (double)(T.c1 * t * t * il2 * il_diag[f]));
+        continue;
+      }
       dFx[i * d + f] = T.c1 * y[f] + T.c2x * x[f] - ex;
       dFy[i * d + f] = T.c1 * x[f] + T.c2z * y[f] + ex;
     }
@@ -996,6 +1185,11 @@ __global__ void kernel_diag_bwd_kernel(const float* __restrict__ Fx, int64_t ldx
 #pragma unroll
     for (int o2 = 16; o2 > 0; o2 >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o2);
     if ((threadIdx.x & 31) == 0 && s != 0.0) atomicAdd(&dhyp[k], s);
+  }
+  if (ARD) {
+    __syncthreads();
+    for (int f = threadIdx.x; f < d; f += blockDim.x)
+      if (dl[f] != 0.0) atomicAdd(&dhyp[4 + f], dl[f]);
   }
 }
 
@@ -1054,12 +1248,20 @@ static size_t bwd_smem(int d) {
 
 static int check_spec(int ta, int da, int tb, int db) {
   auto ok = [](int t, int d) {
+    if (t >= 0 && (t & SVGP_K_ARD)) {                // ARD: the stationary factors with a length scale per feature
+      t &= ~SVGP_K_ARD;
+      if (t != SVGP_K_SE && !is_matern(t)) return false;
+    }
     if (t < 0 || t > SVGP_K_MATERN52 || d < 0) return false;
     if (t == SVGP_K_NONE) return d == 0;
     if (t == SVGP_K_EXPSIN) return d == 1;
     return d >= 1;
   };
   return ok(ta, da) && ok(tb, db) && (da + db) >= 1 && (da + db) <= MAXD;
+}
+// (after check_spec) the flag moves into ard_a / ard_b, so that every comparison of ta / tb sees the base type
+static Spec make_spec(int ta, int da, int tb, int db) {
+  return Spec{ta & ~SVGP_K_ARD, da, tb & ~SVGP_K_ARD, db, (ta & SVGP_K_ARD) != 0, (tb & SVGP_K_ARD) != 0};
 }
 
 }  // namespace svgp
@@ -1089,11 +1291,12 @@ int svgp_kernel_fwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
   SVGP_REQUIRE(!(Kh && !Kl) && !(Kth && !Ktl), "fp16 planes come in hi/lo pairs");
   SVGP_REQUIRE(!(Kh || Kth) || kscale, "fp16 planes need the kscale buffer");
   if (N == 0 || M == 0) return SVGP_OK;
-  Spec sp{type_a, dim_a, type_b, dim_b};
+  const Spec sp = make_spec(type_a, dim_a, type_b, dim_b);
+  const bool ard = sp.ard_a || sp.ard_b;
   cudaStream_t st = (cudaStream_t)stream;
   if (Kh || Kth) {
     if (cudaMemsetAsync(kscale, 0, 8 * sizeof(float), st) != cudaSuccess) return check_launch("svgp_kernel_fwd(memset)");
-    if (type_a == SVGP_K_LINEAR || type_b == SVGP_K_LINEAR) {
+    if (sp.ta == SVGP_K_LINEAR || sp.tb == SVGP_K_LINEAR) {
       int64_t bx = ceil_div(N, 256), bz = ceil_div(M, 256);
       if (bx > 148 * 8) bx = 148 * 8;
       if (bz > 148 * 8) bz = 148 * 8;
@@ -1113,8 +1316,11 @@ int svgp_kernel_fwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
   dim3 grid((unsigned)ntc, (unsigned)gy);
   if (!K && Kh && Kth) {
     // the tcgen05 consumers' operand format only: vectorised builder
-    const bool se44 = type_a == SVGP_K_SE && type_b == SVGP_K_SE && dim_a == 4 && dim_b == 4;
-    if (se44)
+    const bool se44 = sp.ta == SVGP_K_SE && sp.tb == SVGP_K_SE && dim_a == 4 && dim_b == 4;
+    if (ard)
+      kernel_fwd_planes_kernel<false, true><<<grid, THREADS, fwd_smem(dim_a + dim_b) + ARD_SMEM, st>>>(
+          Fx, ldx, N, Fz, ldz, M, sp, hyp, (__half*)Kh, (__half*)Kl, ldkh, (__half*)Kth, (__half*)Ktl, ldkt, kscale);
+    else if (se44)
       kernel_fwd_planes_kernel<true><<<grid, THREADS, fwd_smem(dim_a + dim_b), st>>>(
           Fx, ldx, N, Fz, ldz, M, sp, hyp, (__half*)Kh, (__half*)Kl, ldkh, (__half*)Kth, (__half*)Ktl, ldkt, kscale);
     else
@@ -1126,11 +1332,18 @@ int svgp_kernel_fwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
     // plain fp32 K_nm of a small problem: float64 evaluation, one rounding (the tiled fp32 builder below serves the large ones)
     int64_t blocks = ceil_div(N * M, 256);
     if (blocks > 148 * 32) blocks = 148 * 32;
-    kernel_fwd_f64_kernel<float><<<(unsigned)blocks, 256, 0, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk);
+    if (ard)
+      kernel_fwd_f64_kernel<float, true><<<(unsigned)blocks, 256, MAXD * sizeof(double), st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk);
+    else
+      kernel_fwd_f64_kernel<float><<<(unsigned)blocks, 256, 0, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk);
     return check_launch("svgp_kernel_fwd(f64 evaluation)");
   }
-  kernel_fwd_kernel<<<grid, THREADS, fwd_smem(dim_a + dim_b), st>>>(
-      Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk, (__half*)Kh, (__half*)Kl, ldkh, (__half*)Kth, (__half*)Ktl, ldkt, kscale);
+  if (ard)
+    kernel_fwd_kernel<true><<<grid, THREADS, fwd_smem(dim_a + dim_b) + ARD_SMEM, st>>>(
+        Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk, (__half*)Kh, (__half*)Kl, ldkh, (__half*)Kth, (__half*)Ktl, ldkt, kscale);
+  else
+    kernel_fwd_kernel<<<grid, THREADS, fwd_smem(dim_a + dim_b), st>>>(
+        Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk, (__half*)Kh, (__half*)Kl, ldkh, (__half*)Kth, (__half*)Ktl, ldkt, kscale);
   return check_launch("svgp_kernel_fwd");
 }
 
@@ -1139,10 +1352,15 @@ int svgp_kernel_fwd_f64(const float* Fx, int64_t ldx, int64_t N, const float* Fz
   SVGP_REQUIRE(check_spec(type_a, dim_a, type_b, dim_b), "bad kernel spec");
   SVGP_REQUIRE(Fx && Fz && hyp && K && N >= 0 && M >= 0 && ldk >= M, "bad argument");
   if (N == 0 || M == 0) return SVGP_OK;
-  Spec sp{type_a, dim_a, type_b, dim_b};
+  const Spec sp = make_spec(type_a, dim_a, type_b, dim_b);
+  const bool ard = sp.ard_a || sp.ard_b;
   int64_t blocks = ceil_div(N * M, 256);
   if (blocks > 148 * 32) blocks = 148 * 32;
-  kernel_fwd_f64_kernel<double><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk);
+  if (ard)
+    kernel_fwd_f64_kernel<double, true><<<(unsigned)blocks, 256, MAXD * sizeof(double), (cudaStream_t)stream>>>(
+        Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk);
+  else
+    kernel_fwd_f64_kernel<double><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, K, ldk);
   return check_launch("svgp_kernel_fwd_f64");
 }
 
@@ -1154,7 +1372,8 @@ int svgp_kernel_fwd_i8(const float* Fx, int64_t ldx, int64_t N, const float* Fz,
   SVGP_REQUIRE(ldkh % 8 == 0 && ldkh >= (M + 7) / 8 * 8 && ldkr % 16 == 0 && ldkr >= (M + 7) / 8 * 8, "row pitches: ldkh multiple of 8, ldkr multiple of 16, both >= M rounded up to 8");
   SVGP_REQUIRE((((uintptr_t)Kh | (uintptr_t)Kl | (uintptr_t)Kr | (uintptr_t)Kc) & 15) == 0, "planes need 16-byte alignment");
   if (N == 0 || M == 0) return SVGP_OK;
-  Spec sp{type_a, dim_a, type_b, dim_b};
+  const Spec sp = make_spec(type_a, dim_a, type_b, dim_b);
+  const bool ard = sp.ard_a || sp.ard_b;
   cudaStream_t st = (cudaStream_t)stream;
   float* rmax = scratch;
   float* cmax = scratch + N;
@@ -1171,7 +1390,7 @@ int svgp_kernel_fwd_i8(const float* Fx, int64_t ldx, int64_t N, const float* Fz,
     if (cudaMemsetAsync(Kh, 0, N * ldkh * 2, st) != cudaSuccess || cudaMemsetAsync(Kl, 0, N * ldkh * 2, st) != cudaSuccess)
       return check_launch("svgp_kernel_fwd_i8(memset)");
   }
-  if (type_a == SVGP_K_LINEAR || type_b == SVGP_K_LINEAR) {
+  if (sp.ta == SVGP_K_LINEAR || sp.tb == SVGP_K_LINEAR) {
     int64_t bx = ceil_div(N, 256), bz = ceil_div(M, 256);
     if (bx > 148 * 8) bx = 148 * 8;
     if (bz > 148 * 8) bz = 148 * 8;
@@ -1187,13 +1406,15 @@ int svgp_kernel_fwd_i8(const float* Fx, int64_t ldx, int64_t N, const float* Fz,
   if (gy < 1) gy = 1;
   if (gy > 65535) gy = 65535;
   dim3 grid((unsigned)ntc, (unsigned)gy);
-  const bool se44 = type_a == SVGP_K_SE && type_b == SVGP_K_SE && dim_a == 4 && dim_b == 4;
-  const size_t sm = fwd_smem(dim_a + dim_b);
-#define SVGP_LAUNCH_I8(SE, MX)                                                                                                    \
-  kernel_fwd_i8_kernel<SE, MX><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, (__half*)Kh, (__half*)Kl, ldkh, (int8_t*)Kr, \
-                                                          ldkr, rscale, (int8_t*)Kc, cscale, rmax, cmax, kscale)
-  if (se44) { SVGP_LAUNCH_I8(true, true); SVGP_LAUNCH_I8(true, false); }
-  else { SVGP_LAUNCH_I8(false, true); SVGP_LAUNCH_I8(false, false); }
+  const bool se44 = sp.ta == SVGP_K_SE && sp.tb == SVGP_K_SE && dim_a == 4 && dim_b == 4;
+  const size_t sm = fwd_smem(dim_a + dim_b) + (ard ? ARD_SMEM : 0);
+#define SVGP_LAUNCH_I8(SE, MX, ARD)                                                                                               \
+  kernel_fwd_i8_kernel<SE, MX, ARD><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, (__half*)Kh, (__half*)Kl, ldkh,   \
+                                                               (int8_t*)Kr, ldkr, rscale, (int8_t*)Kc, cscale, rmax, cmax, kscale)
+  if (se44 && ard) { SVGP_LAUNCH_I8(true, true, true); SVGP_LAUNCH_I8(true, false, true); }
+  else if (se44) { SVGP_LAUNCH_I8(true, true, false); SVGP_LAUNCH_I8(true, false, false); }
+  else if (ard) { SVGP_LAUNCH_I8(false, true, true); SVGP_LAUNCH_I8(false, false, true); }
+  else { SVGP_LAUNCH_I8(false, true, false); SVGP_LAUNCH_I8(false, false, false); }
 #undef SVGP_LAUNCH_I8
   return check_launch("svgp_kernel_fwd_i8");
 }
@@ -1204,13 +1425,17 @@ int svgp_kernel_bwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
   SVGP_REQUIRE(check_spec(type_a, dim_a, type_b, dim_b), "bad kernel spec");
   SVGP_REQUIRE(Fx && Fz && hyp && G && N >= 0 && M >= 0, "null input");
   if (N == 0 || M == 0) return SVGP_OK;
-  Spec sp{type_a, dim_a, type_b, dim_b};
-  size_t sm = bwd_smem(dim_a + dim_b);
+  const Spec sp = make_spec(type_a, dim_a, type_b, dim_b);
+  const bool ard = sp.ard_a || sp.ard_b;
+  size_t sm = bwd_smem(dim_a + dim_b) + (ard ? ARD_SMEM : 0);
   cudaStream_t st = (cudaStream_t)stream;
   int64_t ntc = ceil_div(M, TILE), ntr = ceil_div(N, TILE);
   if (dFx) {
     int64_t gx = ntr < 148 * 8 ? ntr : 148 * 8;
-    kernel_bwd_kernel<true><<<(unsigned)gx, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, dFx, nullptr, nullptr);
+    if (ard)
+      kernel_bwd_kernel<true, false, true><<<(unsigned)gx, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, dFx, nullptr, nullptr);
+    else
+      kernel_bwd_kernel<true><<<(unsigned)gx, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, dFx, nullptr, nullptr);
     int rc = check_launch("svgp_kernel_bwd(x)");
     if (rc) return rc;
   }
@@ -1220,12 +1445,19 @@ int svgp_kernel_bwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
     if (gy > ntr) gy = ntr;
     if (gy < 1) gy = 1;
     dim3 grid((unsigned)(ntc < 65535 ? ntc : 65535), (unsigned)gy);
-    const bool se44 = type_a == SVGP_K_SE && type_b == SVGP_K_SE && dim_a == 4 && dim_b == 4 && ntc <= 65535 &&
+    const bool se44 = sp.ta == SVGP_K_SE && sp.tb == SVGP_K_SE && dim_a == 4 && dim_b == 4 && ntc <= 65535 &&
                       !getenv("SVGP_K1_BWD_GENERIC");
-    if (se44)
-      kernel_bwd_z_se44_kernel<<<grid, THREADS, 0, st>>>(Fx, ldx, N, Fz, ldz, M, hyp, G, ldg, dFz, dhyp);
-    else if (is_matern(type_a) || is_matern(type_b))
+    const bool matern = is_matern(sp.ta) || is_matern(sp.tb);
+    if (se44 && ard)
+      kernel_bwd_z_se44_kernel<true><<<grid, THREADS, 0, st>>>(Fx, ldx, N, Fz, ldz, M, hyp, G, ldg, dFz, dhyp, sp);
+    else if (se44)
+      kernel_bwd_z_se44_kernel<<<grid, THREADS, 0, st>>>(Fx, ldx, N, Fz, ldz, M, hyp, G, ldg, dFz, dhyp, sp);
+    else if (matern && ard)
+      kernel_bwd_kernel<false, true, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
+    else if (matern)
       kernel_bwd_kernel<false, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
+    else if (ard)
+      kernel_bwd_kernel<false, false, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
     else
       kernel_bwd_kernel<false><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
     int rc = check_launch("svgp_kernel_bwd(z)");
@@ -1239,10 +1471,14 @@ int svgp_kernel_diag_fwd(const float* Fx, int64_t ldx, const float* Fy, int64_t 
   SVGP_REQUIRE(check_spec(type_a, dim_a, type_b, dim_b), "bad kernel spec");
   SVGP_REQUIRE(Fx && Fy && hyp && kd && N >= 0, "null input");
   if (N == 0) return SVGP_OK;
-  Spec sp{type_a, dim_a, type_b, dim_b};
+  const Spec sp = make_spec(type_a, dim_a, type_b, dim_b);
+  const bool ard = sp.ard_a || sp.ard_b;
   int64_t blocks = ceil_div(N, 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
-  kernel_diag_fwd_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(Fx, ldx, Fy, ldy, N, sp, hyp, kd);
+  if (ard)
+    kernel_diag_fwd_kernel<true><<<(unsigned)blocks, 256, ARD_SMEM, (cudaStream_t)stream>>>(Fx, ldx, Fy, ldy, N, sp, hyp, kd);
+  else
+    kernel_diag_fwd_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(Fx, ldx, Fy, ldy, N, sp, hyp, kd);
   return check_launch("svgp_kernel_diag_fwd");
 }
 
@@ -1252,10 +1488,15 @@ int svgp_kernel_diag_bwd(const float* Fx, int64_t ldx, const float* Fy, int64_t 
   SVGP_REQUIRE(check_spec(type_a, dim_a, type_b, dim_b), "bad kernel spec");
   SVGP_REQUIRE(Fx && Fy && hyp && g && dFx && dFy && dhyp && N >= 0, "null input");
   if (N == 0) return SVGP_OK;
-  Spec sp{type_a, dim_a, type_b, dim_b};
+  const Spec sp = make_spec(type_a, dim_a, type_b, dim_b);
+  const bool ard = sp.ard_a || sp.ard_b;
   int64_t blocks = ceil_div(N, 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
-  kernel_diag_bwd_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(Fx, ldx, Fy, ldy, N, sp, hyp, g, dFx, dFy, dhyp);
+  if (ard)
+    kernel_diag_bwd_kernel<true><<<(unsigned)blocks, 256, ARD_SMEM, (cudaStream_t)stream>>>(Fx, ldx, Fy, ldy, N, sp, hyp, g, dFx,
+                                                                                          dFy, dhyp);
+  else
+    kernel_diag_bwd_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(Fx, ldx, Fy, ldy, N, sp, hyp, g, dFx, dFy, dhyp);
   return check_launch("svgp_kernel_diag_bwd");
 }
 

@@ -19,8 +19,8 @@ import numpy as np
 import torch
 
 from . import ops
-from ._lib import (SVGP_K_COSINE, SVGP_K_EXPSIN, SVGP_K_LINEAR, SVGP_K_MATERN12, SVGP_K_MATERN32, SVGP_K_MATERN52,
-                   SVGP_K_NONE, SVGP_K_SE)
+from ._lib import (SVGP_K_ARD, SVGP_K_COSINE, SVGP_K_EXPSIN, SVGP_K_LINEAR, SVGP_K_MATERN12, SVGP_K_MATERN32,
+                   SVGP_K_MATERN52, SVGP_K_NONE, SVGP_K_SE)
 from .step import LOG_2PI, elbo_terms, svgp_step
 
 
@@ -328,18 +328,48 @@ class productSVGP(mainSVGP):
     over time times a Matern 5/2 kernel over a 3-D position:
 
         productSVGP(Z, dim_a=1, dim_b=3, kind_a="matern32", kind_b="matern52", N_train=N, L=L)
+
+    Automatic relevance determination (ARD): an entry of ``length_scale`` may be a sequence of ``dim_a`` (``dim_b``)
+    floats instead of one float, for the stationary kinds "se" and "matern*".  That block's distance then becomes
+    r^2 = sum_f ((x_f - z_f) / l_f)^2 with one learned length scale per feature column.  The hyper-parameter vector
+    ``GP_hypers_{name}`` is then
+
+        [a_A, l_A, a_B, l_B, l_0, ..., l_{dim_a + dim_b - 1}]        (4 + dim_a + dim_b entries)
+
+    where l_f belongs to feature column f of the [A | B] row.  An ARD block uses its l_f and not its isotropic slot
+    (l_A or l_B, kept at 1.0 with a gradient of 0); an isotropic block uses its slot, and its l_f slots hold 1.0 with a
+    gradient of 0.  With two floats (the default) the vector has 4 entries and the spec is exactly as without ARD.
+    E.g. Matern 3/2 over time times an ARD Matern 5/2 over a 3-D position with one scale per axis:
+
+        productSVGP(Z, dim_a=1, dim_b=3, kind_a="matern32", kind_b="matern52", length_scale=(10.0, [0.5, 0.5, 2.0]),
+                    N_train=N, L=L)
     """
 
     _TYPES = {"se": SVGP_K_SE, "linear": SVGP_K_LINEAR, "cosine": SVGP_K_COSINE, "none": SVGP_K_NONE,
               "matern12": SVGP_K_MATERN12, "matern32": SVGP_K_MATERN32, "matern52": SVGP_K_MATERN52}
+    _ARD_KINDS = ("se", "matern12", "matern32", "matern52")
 
     def __init__(self, initial_inducing_points, dim_a, dim_b, name="prod", jitter=1e-2, N_train=1, L=1, kind_a="se",
                  kind_b="se", amplitude=(1.0, 1.0), length_scale=(1.0, 1.0), fixed_inducing_points=False,
                  fixed_gp_params=False, titsias=False, dtype=torch.float32):
         super().__init__(titsias, fixed_inducing_points, initial_inducing_points, name, jitter, N_train, dtype, L)
         self.dim_a, self.dim_b = dim_a, dim_b
-        self.kinds = (self._TYPES[kind_a], self._TYPES[kind_b])
-        hyp = [amplitude[0], length_scale[0], amplitude[1], length_scale[1]]
+        hyp = [amplitude[0], 1.0, amplitude[1], 1.0]
+        kinds, ard = [], [1.0] * (dim_a + dim_b)
+        for i, (kind, dim, off, ls) in enumerate(((kind_a, dim_a, 0, length_scale[0]), (kind_b, dim_b, dim_a, length_scale[1]))):
+            if np.ndim(ls) == 0:
+                hyp[2 * i + 1] = ls
+                kinds.append(self._TYPES[kind])
+                continue
+            if kind not in self._ARD_KINDS:
+                raise ValueError("one length scale per feature (ARD) needs kind 'se' or 'matern*', not %r" % (kind,))
+            if len(ls) != dim:
+                raise ValueError("block %s has %d features but %d length scales" % ("AB"[i], dim, len(ls)))
+            ard[off:off + dim] = [float(v) for v in ls]
+            kinds.append(self._TYPES[kind] | SVGP_K_ARD)
+        if any(k & SVGP_K_ARD for k in kinds):
+            hyp += ard
+        self.kinds = tuple(kinds)
         _as_param_or_buffer(self, "GP_hypers_{}".format(name), hyp, self.dtype, not fixed_gp_params)
         self._hyp_name = "GP_hypers_{}".format(name)
 
