@@ -104,6 +104,15 @@ def _own_channels(L, group, enabled=True):
     return slice(r * (L // W), (r + 1) * (L // W)), True
 
 
+def syrk_fwd(kop, p, chunk_rows=0):
+    """A_l = sum_i p_il k_i k_i^T, the forward SYRK of the step and of the prediction entry points (predict.py).
+
+    Above M = 2048 the integer path multiplies the three digit-plane pairs of order 4 as well (thirteen pairs): what the ten
+    leave out is what holds the inducing-point gradient at the tolerance there (DESIGN section 7)."""
+    o4 = getattr(kop, "i8", False) and kop.M > 2048
+    return get_backend().syrk(kop, p, impl=IMPL_TC_I8_O4 if o4 else IMPL_AUTO, chunk_rows=chunk_rows)
+
+
 def mm_shared(K, jitter):
     """Channel-independent part of the M x M stage: (K + jI)^-1, its log-det and inverse Cholesky factor (:318-319)."""
     M = K.shape[-1]
@@ -296,10 +305,7 @@ class _SVGPStep(torch.autograd.Function):
         K64 = be.kernel_fwd_f64(spec, Fz32, Fz32, hyp32)
         kappa = be.kernel_diag_fwd(spec, Fx32, Fx32, hyp32)
         p, py, sums = be.rowstats(y32, n32, kappa)
-        # above M = 2048 the forward SYRK multiplies the three digit-plane pairs of order 4 as well (thirteen pairs): what the ten
-        # leave out is what holds the inducing-point gradient at the tolerance there (DESIGN section 7)
-        o4 = getattr(kop, "i8", False) and M > 2048
-        A = be.syrk(kop, p, impl=IMPL_TC_I8_O4 if o4 else IMPL_AUTO, chunk_rows=cfg.get("chunk_rows", 0))
+        A = syrk_fwd(kop, p, chunk_rows=cfg.get("chunk_rows", 0))
         V = be.gemm_tn(kop, py)
         b_total = float(N)
         if group is not None:
