@@ -298,6 +298,15 @@ class _SVGPStep(torch.autograd.Function):
         tc = cfg.get("tc")
         # the tensor-core kernels need tensor-core sized problems (backend.want_tc is the library's own predicate)
         tc = be.want_tc(N, M) if tc is None else (bool(tc) and be.want_tc(N, M))
+        b_total = float(N)
+        if group is not None:
+            # one K_nm format on every rank: the chunked, channel-sharded backward gathers the adjoint operand planes in that
+            # format, so one shard below the tensor-core size takes the whole group to the SIMT kernels.  [rows, 1 - tc]
+            # summed over the ranks: the batch size and the format in one all-reduce and one host read
+            count = torch.tensor([float(N), 0.0 if tc else 1.0], dtype=torch.float64, device=y32.device)
+            _allreduce(count, group)
+            b_total, n_simt = count.tolist()
+            tc = n_simt == 0
 
         # pass A
         kop = be.kernel_fwd(spec, Fx32, Fz32, hyp32, tc=tc)
@@ -307,12 +316,9 @@ class _SVGPStep(torch.autograd.Function):
         p, py, sums = be.rowstats(y32, n32, kappa)
         A = syrk_fwd(kop, p, chunk_rows=cfg.get("chunk_rows", 0))
         V = be.gemm_tn(kop, py)
-        b_total = float(N)
         if group is not None:
-            count = torch.tensor([float(N)], dtype=torch.float64, device=y32.device)
-            for t in (A, V, sums, count):
+            for t in (A, V, sums):
                 _allreduce(t, group)
-            b_total = float(count.item())
         c = N_train / b_total
 
         tri = cfg.get("tri", True)
