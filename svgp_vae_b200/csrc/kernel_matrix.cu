@@ -59,6 +59,8 @@ __device__ __forceinline__ Hyp load_hyp(const float* hyp) {
 __host__ __device__ __forceinline__ bool is_matern(int type) {
   return type == SVGP_K_MATERN12 || type == SVGP_K_MATERN32 || type == SVGP_K_MATERN52;
 }
+// SE and Matern: functions of x - z alone, so their adjoint coefficients have c2z = c2x = -c1
+__host__ __device__ __forceinline__ bool stationary(int type) { return type == SVGP_K_SE || is_matern(type); }
 __device__ __forceinline__ float matern_c(int type) {
   return type == SVGP_K_MATERN12 ? 1.0f : (type == SVGP_K_MATERN32 ? 1.7320508075688772f : 2.2360679774997897f);
 }
@@ -797,20 +799,22 @@ __global__ void __launch_bounds__(THREADS) kernel_fwd_i8_kernel(
 // backward.  Two passes over the same tiles so that neither needs float atomics on N-sized data:
 //   pass X: one block per row tile walks every column tile      -> dFx rows (plain stores)
 //   pass Z: one block per (column tile, row slab) walks its rows -> dFz, dhyp (double atomics,
-//           one flush per block)
-// ACC64 (pass Z of the Matern factors): the per-tile fp32 partials are folded into double across the row tiles and the
-// flush  dz_f = sum c1 x_f + z_f sum c2z  (which cancels: c2z = -c1) is done in double, as in kernel_bwd_z_se44_kernel
+//           one flush per block); the per-tile fp32 partials are folded into double across the row tiles
+// Stationary factors (SE, Matern: c2 = -c1) sum  c1 (other_f - own_f)  per entry: dz_f = sum c1 (x_f - z_f) and
+// dx_f = sum c1 (z_f - x_f).  The moment form  sum c1 x_f + z_f sum c2z  cancels in fp32 for offset features (time
+// stamps at 1e4 with l = 10: up to 4e-5 of dz, 7e-5 of dx); LINEAR and COSINE keep it (c2 is not -c1 there).
 // ARD: the coefficients are those of the scaled coordinates (factor_adjoint), the phase-2 sums run on the unscaled
 // features, and the flush multiplies by il_f^2.  Pass Z also sums  c1 (x_f - z_f)^2  per entry for every feature of an
 // ARD block (fp32 per tile, folded into double): dl_f = il_f^3 times that.  (Per-column moments sum c1 x^2, sum c1 x,
 // sum c1 would cancel by orders of magnitude in fp32 for offset features such as time stamps.)
 // ------------------------------------------------------------------------------------------
-template <bool PASS_X, bool ACC64 = false, bool ARD = false>
-__global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
+// (three blocks per SM: up to 85 registers -- with no minimum ptxas picked 64 and spilled in the fp32 X pass)
+template <bool PASS_X, bool ARD = false>
+__global__ void __launch_bounds__(THREADS, 3) kernel_bwd_kernel(
     const float* __restrict__ Fx, int64_t ldx, int64_t N, const float* __restrict__ Fz, int64_t ldz, int64_t M,
     Spec sp, const float* __restrict__ hyp, const float* __restrict__ G, int64_t ldg, float* __restrict__ dFx,
     double* __restrict__ dFz, double* __restrict__ dhyp) {
-  static_assert(!(PASS_X && ACC64), "ACC64 is a Z-pass variant");
+  constexpr bool ACC64 = !PASS_X;
   extern __shared__ float smem[];
   const int d = sp.da + sp.db, dp = d | 1;
   float* xs = smem;
@@ -898,11 +902,12 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
           const int f = fg + 4 * q;
           if (f < d) {
             const float* cmat = (f < sp.da) ? c1a : c1b;
+            const float own_f = stationary(f < sp.da ? sp.ta : sp.tb) ? (PASS_X ? xs : zs)[o * dp + f] : 0.f;
             float s = 0.f;
             if (PASS_X) {
-              for (int k = 0; k < TILE; ++k) s = fmaf(cmat[o * (TILE + 1) + k], zs[k * dp + f], s);
+              for (int k = 0; k < TILE; ++k) s = fmaf(cmat[o * (TILE + 1) + k], zs[k * dp + f] - own_f, s);
             } else {
-              for (int k = 0; k < TILE; ++k) s = fmaf(cmat[k * (TILE + 1) + o], xs[k * dp + f], s);
+              for (int k = 0; k < TILE; ++k) s = fmaf(cmat[k * (TILE + 1) + o], xs[k * dp + f] - own_f, s);
             }
             if (ACC64) acc64[q] += (double)s;
             else acc[q] += s;
@@ -940,15 +945,16 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
         const int f = fg + 4 * q;
         if (f >= d) continue;
         bool inA = f < sp.da;
+        const bool diff = stationary(inA ? sp.ta : sp.tb);     // phase 2 already summed c1 (other_f - own_f)
         if (ACC64) {
-          double v = acc64[q] + own64[inA ? 0 : 1] * (double)self[f];
+          double v = acc64[q] + (diff ? 0.0 : own64[inA ? 0 : 1] * (double)self[f]);
           if (inA && f == 0 && sp.ta == SVGP_K_EXPSIN) v += own64[2];
           if (!inA && f == sp.da && sp.tb == SVGP_K_EXPSIN) v += own64[3];
           if (ARD) v *= (double)il[f] * (double)il[f];
           if (go < M) atomicAdd(&dFz[go * d + f], v);
           continue;
         }
-        float v = acc[q] + own[o * 4 + (inA ? 0 : 1)] * self[f];
+        float v = acc[q] + (diff ? 0.f : own[o * 4 + (inA ? 0 : 1)] * self[f]);
         // EXPSIN contributes only through its single feature (the first of its block)
         if (inA && f == 0 && sp.ta == SVGP_K_EXPSIN) v += own[o * 4 + 2];
         if (!inA && f == sp.da && sp.tb == SVGP_K_EXPSIN) v += own[o * 4 + 3];
@@ -988,7 +994,8 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_kernel(
 
 // Z pass specialised for the product of two 4-feature SE factors (the SWEEP kernel; the generic pass above spends
 // ~20 ns per 1000 entries on run-time factor dispatch, a second distance evaluation and four double adds per entry).
-// With c = g k:  dz_f = (sum_i c x_if - z_f sum_i c) / l^2,  dl = sum c r2 / l^3,  damp = 2 sum c / amp  per block --
+// With c = g k:  dz_f = sum_i c (x_if - z_f) / l^2,  dl = sum c r2 / l^3,  damp = 2 sum c / amp  per block (the per-entry
+// differences d_f, not sum c x_f - z_f sum c: that cancels in fp32 for offset features such as time stamps) --
 // a thread owns one inducing point (features in registers) and 16 of the 64 datapoints of a tile, the datapoint
 // features are broadcast float4 loads, g is read in coalesced 128-byte rows; one float partial per tile, folded into
 // double per thread (the hyper-parameter sums cancel heavily), one double atomic per (column, feature) per block.
@@ -1002,7 +1009,7 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
     double* __restrict__ dhyp, Spec sp) {
   constexpr int NS = ARD ? 17 : 11, NH = ARD ? 12 : 4;   // partials per thread, dhyp slots
   __shared__ __align__(16) float xs[TILE * 8];
-  __shared__ double red[4][TILE][NS];            // per row group: 8 feature sums, sum c, sum c r2a, sum c r2b (ARD: 8 x sum c d_f^2)
+  __shared__ double red[4][TILE][NS];            // per row group: 8 x sum c d_f, sum c, sum c r2a, sum c r2b (ARD: 8 x sum c d_f^2)
   const Hyp h = load_hyp(hyp);
   const int c = threadIdx.x % TILE, rg = threadIdx.x / TILE;
   const int64_t ntr = (N + TILE - 1) / TILE;
@@ -1047,8 +1054,8 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
 #pragma unroll
         for (int f = 0; f < 8; ++f) ex = fmaf(cf[f], sq[f], ex);
         const float ck = g * amp2 * exp2f(ex);
-        t[0] = fmaf(ck, xa.x, t[0]); t[1] = fmaf(ck, xa.y, t[1]); t[2] = fmaf(ck, xa.z, t[2]); t[3] = fmaf(ck, xa.w, t[3]);
-        t[4] = fmaf(ck, xb.x, t[4]); t[5] = fmaf(ck, xb.y, t[5]); t[6] = fmaf(ck, xb.z, t[6]); t[7] = fmaf(ck, xb.w, t[7]);
+        t[0] = fmaf(ck, d0, t[0]); t[1] = fmaf(ck, d1, t[1]); t[2] = fmaf(ck, d2, t[2]); t[3] = fmaf(ck, d3, t[3]);
+        t[4] = fmaf(ck, e0, t[4]); t[5] = fmaf(ck, e1, t[5]); t[6] = fmaf(ck, e2, t[6]); t[7] = fmaf(ck, e3, t[7]);
         t[8] += ck;
 #pragma unroll
         for (int f = 0; f < 8; ++f) t[9 + f] = fmaf(ck, sq[f], t[9 + f]);
@@ -1057,8 +1064,8 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
       const float ra = fmaf(d3, d3, fmaf(d2, d2, fmaf(d1, d1, d0 * d0)));
       const float rb = fmaf(e3, e3, fmaf(e2, e2, fmaf(e1, e1, e0 * e0)));
       const float ck = g * amp2 * exp2f(fmaf(ca, ra, cb * rb));
-      t[0] = fmaf(ck, xa.x, t[0]); t[1] = fmaf(ck, xa.y, t[1]); t[2] = fmaf(ck, xa.z, t[2]); t[3] = fmaf(ck, xa.w, t[3]);
-      t[4] = fmaf(ck, xb.x, t[4]); t[5] = fmaf(ck, xb.y, t[5]); t[6] = fmaf(ck, xb.z, t[6]); t[7] = fmaf(ck, xb.w, t[7]);
+      t[0] = fmaf(ck, d0, t[0]); t[1] = fmaf(ck, d1, t[1]); t[2] = fmaf(ck, d2, t[2]); t[3] = fmaf(ck, d3, t[3]);
+      t[4] = fmaf(ck, e0, t[4]); t[5] = fmaf(ck, e1, t[5]); t[6] = fmaf(ck, e2, t[6]); t[7] = fmaf(ck, e3, t[7]);
       t[8] += ck; t[9] = fmaf(ck, ra, t[9]); t[10] = fmaf(ck, rb, t[10]);
     }
 #pragma unroll
@@ -1074,7 +1081,7 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
 #pragma unroll
     for (int f = 0; f < 8; ++f) {
       const double l = ard_len(hyp, sp, h, f), il2 = 1.0 / (l * l);
-      atomicAdd(&dFz[gc * 8 + f], (s[f] - (double)z[f] * s[8]) * il2);
+      atomicAdd(&dFz[gc * 8 + f], s[f] * il2);
       dl[f] = s[9 + f] * il2 / l;
     }
     red[0][c][0] = 2.0 * s[8] / h.amp_a; red[0][c][1] = sp.ard_a ? 0.0 : dl[0] + dl[1] + dl[2] + dl[3];
@@ -1090,7 +1097,7 @@ __global__ void __launch_bounds__(THREADS) kernel_bwd_z_se44_kernel(
     for (int q = 0; q < NS; ++q) s[q] = red[0][c][q] + red[1][c][q] + red[2][c][q] + red[3][c][q];
     const double ila = 1.0 / ((double)h.len_a * h.len_a), ilb = 1.0 / ((double)h.len_b * h.len_b);
 #pragma unroll
-    for (int f = 0; f < 8; ++f) atomicAdd(&dFz[gc * 8 + f], (s[f] - (double)z[f] * s[8]) * (f < 4 ? ila : ilb));
+    for (int f = 0; f < 8; ++f) atomicAdd(&dFz[gc * 8 + f], s[f] * (f < 4 ? ila : ilb));
     red[0][c][0] = 2.0 * s[8] / h.amp_a; red[0][c][1] = s[9] * ila / h.len_a;
     red[0][c][2] = 2.0 * s[8] / h.amp_b; red[0][c][3] = s[10] * ilb / h.len_b;
   } else if (rg == 0) {
@@ -1244,6 +1251,12 @@ static size_t fwd_smem(int d) {
 static size_t bwd_smem(int d) {
   int dp = d | 1;
   return sizeof(float) * (2 * TILE * dp + 2 * TILE * (TILE + 1) + 4 * TILE + 4 * TILE + 4);
+}
+
+// the backward's layout passes the 48 KB default of dynamic shared memory from d = 26 features on (d = 32: 52 KB)
+template <typename F>
+static void allow_smem(F* kernel, size_t bytes) {
+  if (bytes > 48 * 1024) cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
 static int check_spec(int ta, int da, int tb, int db) {
@@ -1430,10 +1443,12 @@ int svgp_kernel_bwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
   size_t sm = bwd_smem(dim_a + dim_b) + (ard ? ARD_SMEM : 0);
   cudaStream_t st = (cudaStream_t)stream;
   int64_t ntc = ceil_div(M, TILE), ntr = ceil_div(N, TILE);
+  allow_smem(ard ? kernel_bwd_kernel<true, true> : kernel_bwd_kernel<true>, sm);
+  allow_smem(ard ? kernel_bwd_kernel<false, true> : kernel_bwd_kernel<false>, sm);
   if (dFx) {
     int64_t gx = ntr < 148 * 8 ? ntr : 148 * 8;
     if (ard)
-      kernel_bwd_kernel<true, false, true><<<(unsigned)gx, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, dFx, nullptr, nullptr);
+      kernel_bwd_kernel<true, true><<<(unsigned)gx, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, dFx, nullptr, nullptr);
     else
       kernel_bwd_kernel<true><<<(unsigned)gx, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, dFx, nullptr, nullptr);
     int rc = check_launch("svgp_kernel_bwd(x)");
@@ -1447,17 +1462,12 @@ int svgp_kernel_bwd(const float* Fx, int64_t ldx, int64_t N, const float* Fz, in
     dim3 grid((unsigned)(ntc < 65535 ? ntc : 65535), (unsigned)gy);
     const bool se44 = sp.ta == SVGP_K_SE && sp.tb == SVGP_K_SE && dim_a == 4 && dim_b == 4 && ntc <= 65535 &&
                       !getenv("SVGP_K1_BWD_GENERIC");
-    const bool matern = is_matern(sp.ta) || is_matern(sp.tb);
     if (se44 && ard)
       kernel_bwd_z_se44_kernel<true><<<grid, THREADS, 0, st>>>(Fx, ldx, N, Fz, ldz, M, hyp, G, ldg, dFz, dhyp, sp);
     else if (se44)
       kernel_bwd_z_se44_kernel<<<grid, THREADS, 0, st>>>(Fx, ldx, N, Fz, ldz, M, hyp, G, ldg, dFz, dhyp, sp);
-    else if (matern && ard)
-      kernel_bwd_kernel<false, true, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
-    else if (matern)
-      kernel_bwd_kernel<false, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
     else if (ard)
-      kernel_bwd_kernel<false, false, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
+      kernel_bwd_kernel<false, true><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
     else
       kernel_bwd_kernel<false><<<grid, THREADS, sm, st>>>(Fx, ldx, N, Fz, ldz, M, sp, hyp, G, ldg, nullptr, dFz, dhyp);
     int rc = check_launch("svgp_kernel_bwd(z)");

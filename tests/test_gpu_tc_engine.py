@@ -7,24 +7,27 @@ from svgp_vae_b200.backend import IMPL_SIMT, Kop
 
 pytestmark = pytest.mark.gpu
 SPEC = (1, 4, 1, 4)
+# LINEAR x COSINE on [16 | 16]: K has negative entries (kscale[6] = 0: no one-signed truncation-bias correction)
+SIGNED = (3, 16, 4, 16)
 
 
-def _setup(be, N, M, L, seed=0):
+def _setup(be, N, M, L, seed=0, spec=SPEC, i8=False):
     g = torch.Generator(device="cuda").manual_seed(seed)
-    Fx = torch.randn(N, 8, generator=g, device="cuda")
-    Fz = torch.randn(M, 8, generator=g, device="cuda")
+    Fx = torch.randn(N, spec[1] + spec[3], generator=g, device="cuda")
+    Fz = torch.randn(M, spec[1] + spec[3], generator=g, device="cuda")
     hyp = torch.ones(4, device="cuda")
-    kop = be.kernel_fwd(SPEC, Fx, Fz, hyp, tc=True, i8=False)
+    kop = be.kernel_fwd(spec, Fx, Fz, hyp, tc=True, i8=i8)
+    assert float(kop.kscale[6]) == (0.0 if spec == SIGNED else 1.0)
     K64 = kop.value().double()
     W = torch.randn(N, L, generator=g, device="cuda")
     return kop, K64, W, g
 
 
 @pytest.mark.parametrize("shape", [(4096, 256, 3), (3000, 200, 2), (8192, 384, 2), (2500, 1024, 1)])
-def test_tc_syrk(cuda_backend, shape):
+def test_tc_syrk(cuda_backend, shape, spec=SPEC):
     be = cuda_backend
     N, M, L = shape
-    kop, K64, W, g = _setup(be, N, M, L)
+    kop, K64, W, g = _setup(be, N, M, L, spec=spec)
     ref = torch.einsum('il,ia,ib->lab', W.double(), K64, K64)
     # the tensor core accumulates with truncation: the bias grows ~2.7e-8 per MMA of a chain (measured,
     # profiles/r01_accuracy.md), so short chains (chunk_rows=128 -> 24 MMAs) reach fp32-level accuracy and
@@ -39,6 +42,11 @@ def test_tc_syrk(cuda_backend, shape):
     Wp = torch.exp(torch.empty(N, L, device="cuda").uniform_(-4.6, 9.2, generator=g))
     refp = torch.einsum('il,ia,ib->lab', Wp.double(), K64, K64)
     assert rel_err(be.syrk(kop, Wp), refp) < 3e-5
+
+
+@pytest.mark.parametrize("shape", [(4096, 256, 3), (2500, 1024, 1)])
+def test_tc_syrk_signed(cuda_backend, shape):
+    test_tc_syrk(cuda_backend, shape, SIGNED)
 
 
 @pytest.mark.parametrize("shape", [(9000, 256, 1), (20000, 384, 3), (20000, 384, 4), (70000, 1024, 2)])
@@ -58,10 +66,10 @@ def test_tc_syrk_superchunks(cuda_backend, shape, monkeypatch):
 
 
 @pytest.mark.parametrize("shape", [(4096, 256, 3), (3000, 200, 2), (2304, 1024, 2)])
-def test_tc_rowquad_scaled(cuda_backend, shape):
+def test_tc_rowquad_scaled(cuda_backend, shape, spec=SPEC, i8=False):
     be = cuda_backend
     N, M, L = shape
-    kop, K64, W, g = _setup(be, N, M, L, seed=1)
+    kop, K64, W, g = _setup(be, N, M, L, seed=1, spec=spec, i8=i8)
     S = torch.randn(L, M, M, generator=g, device="cuda", dtype=torch.float64)
     S = (S + S.transpose(1, 2)).contiguous()
     S[0] *= 1e4                                      # per-matrix scaling of the fp16 planes
@@ -81,6 +89,12 @@ def test_tc_rowquad_scaled(cuda_backend, shape):
     assert rel_err(out, 2 * refo) < 3e-5
     out1, dots1 = be.scaled_gemm(kop, W, S, ndot=1)
     assert rel_err(out1, refo) < 3e-5 and rel_err(dots1[:, 0], ref[:, 0]) < 3e-5
+
+
+@pytest.mark.parametrize("shape", [(4096, 256, 3), (2304, 1024, 2)])
+def test_tc_rowquad_scaled_signed(cuda_backend, shape):
+    """The row quads and the scaled GEMM on the fp16 row planes of the integer builder (the step's default format)."""
+    test_tc_rowquad_scaled(cuda_backend, shape, SIGNED, i8=True)
 
 
 @pytest.mark.parametrize("shape", [(4096, 256, 3), (3000, 200, 64), (2304, 1024, 70), (2500, 384, 300)])

@@ -227,3 +227,34 @@ def test_oracle_titsias_matches_reference_source():
     _, _, mu_hat, A_hat = sb.approximate_posterior_params(x, y, nz)
     L2, _ = sb.variational_loss(x, y, nz, mu_hat, A_hat)
     assert _close(L2, gold["ball_titsias/L2"], 1e-10)
+
+
+def test_parity_fullsize_kinds_factor_formulas():
+    """tests/probes/parity_fullsize_kinds.py builds K_nm, K_mm and kappa from per-block formulas of its own (no (N, M, d)
+    tensor, differences rather than the |x|^2 + |z|^2 - 2 x.z expansion): they must equal the oracle formulas
+    (oracle_backend / matern_oracle.kernel_value, oracle/tfp_kernels) on every case's features, the time column offset
+    by 1e4 included."""
+    import sys
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "probes"))
+    import matern_oracle as mo
+    import oracle_backend as ob
+    import parity_fullsize_kinds as pk
+    rel = lambda a, b: float((a - b).abs().max() / b.abs().max())
+    for case, c in pk.CASES.items():
+        X, Z = pk.features(case, 300, 70, "cpu", 5)
+        hyp = torch.tensor([0.9, c["ls"][0], 1.1, c["ls"][1]], dtype=torch.float64)
+        spec = pk.spec_of(c["kinds"], c["dims"])
+        X64, Z64 = X.double(), Z.double()
+        assert rel(pk.kern64(X64, Z64, hyp, c["kinds"], c["dims"]), mo.kernel_value(spec, X, Z, hyp)) < 1e-12, case
+        assert rel(pk.kern64(Z64, Z64, hyp, c["kinds"], c["dims"]), mo.kernel_value(spec, Z, Z, hyp)) < 1e-12, case
+        assert rel(pk.kdiag64(X64, hyp, c["kinds"], c["dims"]), mo.kernel_value(spec, X, X, hyp, pairwise=False)) < 1e-12, case
+        if "matern32" not in c["kinds"]:
+            assert rel(pk.kern64(X64, Z64, hyp, c["kinds"], c["dims"]), ob.kernel_value(spec, X, Z, hyp)) < 1e-12, case
+    # each factor against tfp_kernels directly, the offset time column included
+    X, Z = pk.features("time_m32_se", 200, 50, "cpu", 3)
+    X64, Z64 = X.double(), Z.double()
+    ten = torch.tensor(10.0, dtype=torch.float64)
+    assert rel(pk.factor64("se", X64[:, :1], Z64[:, :1], 1.0, ten), tfk.ExponentiatedQuadratic(1.0, ten).matrix(X64[:, :1], Z64[:, :1])) < 1e-12
+    assert rel(pk.factor64("se", X64, Z64, 1.3, ten), tfk.ExponentiatedQuadratic(1.3, ten).matrix(X64, Z64)) < 1e-12
+    assert rel(pk.factor64("matern32", X64[:, :1], Z64[:, :1], 1.0, ten), mo.MaternThreeHalves(1.0, ten).matrix(X64[:, :1], Z64[:, :1])) < 1e-12
+    assert rel(pk.factor64("linear", X64, Z64, 1.0, 1.0), tfk.Linear().matrix(X64, Z64)) < 1e-12
